@@ -18,6 +18,8 @@ reference from oracle/_ref (bytecode compiled by oracle/build_ref.py) on the hos
 (`kind: "reference"`), else the oracle port (`kind: "port"`); its config line states the batch it really ran.
 """
 import argparse
+import atexit
+import contextlib
 import json
 import os
 import subprocess
@@ -30,6 +32,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: no bytecode caches next to the sources
 
 METRIC = 'impflow_train_samples_per_sec'
 UNIT = 'samples/s'
@@ -178,8 +181,14 @@ class ClockSampler(object):
             self.proc = subprocess.Popen(['nvidia-smi', '-i', str(self.gpu), '--query-gpu=' + self.QUERY,
                                           '--format=csv,noheader,nounits', '-lms', '400'],
                                          stdout=open(self.path, 'w'), stderr=subprocess.DEVNULL)
+            atexit.register(self._reap)         # also when the run fails before stop(): no poller outlives it
         except Exception:
             self.proc = None
+
+    def _reap(self):
+        if self.proc is not None and self.proc.poll() is None:
+            self.proc.kill()
+            self.proc.wait()
 
     def stop(self):
         out = {'sm_mhz': None, 'sm_max_mhz': None, 'reasons': []}
@@ -241,21 +250,51 @@ def synthetic_batch(wl, batch, gen):
     return torch.rand(batch, c, h, w, generator=gen), y
 
 
-def loss_of(model, wl, x, y):
+def loss_of(model, wl, x, y, outputs=None):
     """The training objective of the three script families (train_img.py:517-549, train_tabular.py:398-407 /
-    train_toy.py:108-116, train_classification.py:357-359)."""
+    train_toy.py:108-116, train_classification.py:357-359).  `outputs`, when given, receives copies of what the model
+    returned: the logits, or the latent `z` and the log-determinant `logdet`."""
     kind = wl.get('kind')
     if kind == 'cls':
-        return torch.nn.functional.cross_entropy(model(x), y, reduction='sum')
+        logits = model(x)
+        if outputs is not None:
+            outputs['logits'] = logits.detach().clone()
+        return torch.nn.functional.cross_entropy(logits, y, reduction='sum')
     if kind == 'mlp':
         z, dlogp = model(x, torch.zeros(x.shape[0], 1, device=x.device))
+        if outputs is not None:
+            outputs['z'], outputs['logdet'] = z.detach().clone(), dlogp.detach().clone()
         logpz = std_normal_logprob(z).reshape(z.size(0), -1).sum(1, keepdim=True)
         return -(logpz - dlogp).mean()
     n_dims = int(np.prod(wl['input']))
     z, dlogp = model(x, 0)
+    if outputs is not None:
+        outputs['z'], outputs['logdet'] = z.detach().clone(), dlogp.detach().clone()
     logpz = std_normal_logprob(z).reshape(z.size(0), -1).sum(1, keepdim=True)
     logpx = logpz - dlogp - np.log(256) * n_dims
     return -torch.mean(logpx) / n_dims / np.log(2)
+
+
+DUMP_BYTES = 64 * 1000 * 1000
+DUMP_CAP = {'params': 6000000, 'grads': 6000000}      # elements; every other array: 1000000
+
+
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: every array as out_dir/<name>.npy in float32 (float64 stays float64).  An array longer than its
+    cap is replaced by a sample of its flattened elements at fixed positions (seed 0, so the same positions in every run
+    of one configuration, and the same ones in `params` and `grads`); the directory stays under DUMP_BYTES."""
+    out = {}
+    for name, t in arrays.items():
+        a = t.detach().cpu().numpy()
+        a = a if a.dtype == np.float64 else a.astype(np.float32)
+        cap = DUMP_CAP.get(name, 1000000)
+        if a.size > cap:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        out[name] = a
+    assert sum(a.nbytes for a in out.values()) <= DUMP_BYTES - 4096 * len(out)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def run_reference_impl(wl_name, steps, warmup, batch, threads=None):
@@ -533,6 +572,10 @@ def main():
                     help='N > 1: the Russian-roulette term counts n are drawn from one seed on every rank (equal work '
                          'per rank; each rank\'s estimate stays unbiased, probes and data stay per-rank) or per rank '
                          '(what the reference\'s DataParallel threads do; the step then waits for the unluckiest rank)')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write what the last of them computed (loss, model outputs, updated '
+                         'parameters, gradients) as DIR/<name>.npy; the inputs are seeded, so two builds run with the '
+                         'same arguments can be compared output for output')
     args = ap.parse_args()
 
     rank = int(os.environ.get('RANK', 0))
@@ -553,6 +596,8 @@ def main():
               'probe_mode': args.probe_mode, 'roulette_draws': args.roulette if world > 1 else 'single rank'}
 
     if args.impl == 'reference':
+        if args.dump_outputs:
+            ap.error('--dump-outputs writes the outputs of the GPU path (--impl b200)')
         if rank != 0:
             return
         # a bounded sample of the workload per step, stated in the line's own config: the metric is per sample
@@ -576,6 +621,8 @@ def main():
                 'solver_iterations': solver}
         print(json.dumps(line))
         return
+    if args.steps < 1:
+        ap.error('--steps: at least one timed step')
 
     import torch.distributed as dist
     assert torch.cuda.is_available(), 'bench.py --impl b200 needs a GPU (there is no CPU fallback)'
@@ -596,7 +643,8 @@ def main():
             os.close(saved_fd)
     import __graft_entry__
     if rank == 0:
-        __graft_entry__.build()
+        with contextlib.redirect_stdout(sys.stderr):      # stdout carries the JSON line only
+            __graft_entry__.build()
     if world > 1:
         dist.barrier()
     import impflow_b200 as pkg
@@ -665,9 +713,9 @@ def main():
     flush = torch.empty(64 * 1024 * 1024, device=dev, dtype=torch.float32)
     blocks = [m for m in model.modules() if isinstance(m, pkg.layers.imBlock)]
 
-    def step(x, y=None):
+    def step(x, y=None, outputs=None):
         bucket.zero()
-        loss = loss_of(model, wl, x, y)
+        loss = loss_of(model, wl, x, y, outputs)
         loss.backward()
         bucket.allreduce_mean()
         opt.step()
@@ -722,13 +770,14 @@ def main():
     torch.cuda.nvtx.range_push('timed')
     if os.environ.get('IMPFLOW_PROFILER_API', '') == '1':      # ncu --profile-from-start off: every thread's launches
         torch.cuda.cudart().cudaProfilerStart()
+    dumped = {} if args.dump_outputs and rank == 0 else None
     ev0.record()
     step_evs = [ev0]
     for i_ in range(args.steps):
         if trace:
             sys.stderr.write('[timed step %d] t=%.3f\n' % (i_, time.perf_counter()))
         flush.zero_()
-        step(x_dev, y_dev)
+        loss_last = step(x_dev, y_dev, dumped if i_ == args.steps - 1 else None)
         step_evs.append(torch.cuda.Event(enable_timing=True))
         step_evs[-1].record()
         solves += 2 * len(blocks) * batch
@@ -743,6 +792,14 @@ def main():
     per_step_ms = [round(a.elapsed_time(b), 2) for a, b in zip(step_evs[:-1], step_evs[1:])]
     launches = pkg._cabi.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if dumped is not None:
+        # besides the model outputs: the last timed step's loss, the parameters its optimiser step left and the
+        # gradients it applied (taken now: the passes below train on)
+        dumped['loss'] = loss_last.detach().reshape(1)
+        dumped['params'] = torch.cat([p.detach().reshape(-1) for p in params])
+        dumped['grads'] = torch.cat([g.reshape(-1) for g in bucket.views])
+        write_outputs(args.dump_outputs, dumped)
+        dumped = None
 
     # ---------------- instrumented pass (NOT the timed region): the same K steps again with the per-launch shape
     # recorder and CUDA events around every solve switched on.  The recorder costs host time per launch, and the step
