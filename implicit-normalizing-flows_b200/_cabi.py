@@ -59,8 +59,6 @@ SIGNATURES = {
                                 _ll, _ll, _i, _i, _i, _c_fp, _c_fp, _c_fp]),
     'impflow_branch3_tc': (_i, [_c_fp, _ll] + [_c_fp] * 13 + [_ll, _ll, _i, _i, _i, _c_fp, _c_fp, _c_fp]),
     'impflow_chain23_parts': (_i, [_i]),
-    'impflow_chain23_set_multicast': (_i, [_i]),
-    'impflow_broyden_set_chunk': (_i, [_i]),
     'impflow_chain23_tc': (_i, [_c_fp, _c_fp, _ll] + [_c_fp] * 8 + [_ll, _ll, _ll, _i, _i, _i, _c_fp, _c_fp]),
     'impflow_conv3_set_chain23': (_i, [_i]),
     'impflow_conv3_set_chain23_a32': (_i, [_i]),
@@ -77,7 +75,6 @@ SIGNATURES = {
     'impflow_wgrad_tc_workspace_floats': (ctypes.c_size_t, [_ll, _i, _i]),
     'impflow_wgrad_tc': (_i, [_c_fp, _c_fp, _ll, _c_fp, _c_fp, _ll, _c_fp, _ll, _i, _ll, _i, _i, _c_fp, _c_fp]),
     'impflow_gemm_tc_splits': (_i, [_ll, _i, _i]),
-    'impflow_gemm_tc_set_wide_tiles': (_i, [_i]),
     'impflow_gemm_tc_set_tma_store': (_i, [_i]),
     'impflow_gemm_tc_set_pair': (_i, [_i]),
     'impflow_set_pdl': (_i, [_i]),

@@ -163,24 +163,19 @@ __global__ void k_begin(const float* __restrict__ x0, const float* __restrict__ 
 }
 
 // ------------------------------------------------------------------------------------------
-// rank-1 update, cluster per sample.  VEC = 4 (float4 path, d % 4 == 0) or 1.
+// rank-1 update, cluster per sample.  VEC = 4 (float4 path, d % 4 == 0) or 1.  Two CTAs of 8 warps per SM.
 // dynamic smem: sdx[SL] sdg[SL] sgn[SL] | wsum[3*T][kWarps] | part0[3*T] part1[2] | tot[3*T+2]
 // ------------------------------------------------------------------------------------------
-template <int LD>
-__device__ __forceinline__ float4 ld_hist(const float4* p) {
-  return LD == 0 ? __ldg(p) : __ldcg(p);
-}
-
-// NT threads per CTA (256: two CTAs of 8 warps per SM; 512: two CTAs of 16 warps), LD: history loads through the
-// read-only path (0) or L1-bypassing (1)
-template <int VEC, int NT, int LD>
-__global__ void __launch_bounds__(NT, 2)
+template <int VEC>
+__global__ void __launch_bounds__(kThreads, 2)
 k_update(float* __restrict__ x_old, const float* __restrict__ g_old, const float* __restrict__ xn,
          const float* __restrict__ gn, float* __restrict__ Ut, float* __restrict__ Vt,
          float* __restrict__ low_x, float* __restrict__ low_g, const impflow_broyden_state* st, long long d,
          int T, int SL, int expect_nstep) {
-  constexpr int kThreads = NT;
-  constexpr int kWarps = NT / 32;
+  // local copies of the block shape: without them nvcc assigns two accumulators other registers than in the build
+  // whose speed profiles/ records (same instructions, same register count)
+  constexpr int kThreads = impflow::kThreads;
+  constexpr int kWarps = impflow::kWarps;
   const int do_update = st->do_update;
   const int new_low = st->new_lowest;
   if (!do_update && !new_low) return;  // uniform over the whole grid
@@ -208,7 +203,7 @@ k_update(float* __restrict__ x_old, const float* __restrict__ g_old, const float
 
   // ---- phase 0: deltas into smem, best-iterate copy (:159-162, :94-99) ----
   if (VEC == 4) {
-    constexpr int UN = NT >= 512 ? 2 : 4;       // 16 (8) independent loads per thread in flight
+    constexpr int UN = 4;       // 16 independent loads per thread in flight
     for (int i0 = tid * 4; i0 < len; i0 += kThreads * 4 * UN) {
       float4 xo[UN], xv[UN], go[UN], gv[UN];
 #pragma unroll
@@ -268,15 +263,15 @@ k_update(float* __restrict__ x_old, const float* __restrict__ g_old, const float
     if (VEC == 4) {
       // the kernel is bound by load latency, not by DRAM bytes: 16 independent 16-byte loads per thread in flight
       // (same per-thread summation order as a plain loop)
-      constexpr int UN = NT >= 512 ? 4 : 8;
+      constexpr int UN = 8;
       for (int i0 = tid * 4; i0 < len; i0 += kThreads * 4 * UN) {
         float4 u4[UN], v4[UN];
 #pragma unroll
         for (int q = 0; q < UN; ++q) {
           const int i = i0 + q * kThreads * 4;
           if (i < len) {
-            u4[q] = ld_hist<LD>(reinterpret_cast<const float4*>(uj + i));
-            v4[q] = ld_hist<LD>(reinterpret_cast<const float4*>(vj + i));
+            u4[q] = __ldg(reinterpret_cast<const float4*>(uj + i));
+            v4[q] = __ldg(reinterpret_cast<const float4*>(vj + i));
           }
         }
 #pragma unroll
@@ -339,13 +334,13 @@ k_update(float* __restrict__ x_old, const float* __restrict__ g_old, const float
     }
     int j = 0;
     if (VEC == 4) {
-      constexpr int UJ = NT >= 512 ? 4 : 8;       // 16 (8) independent loads in flight per thread; accumulation order over j unchanged
+      constexpr int UJ = 8;       // 16 independent loads in flight per thread; accumulation order over j unchanged
       for (; j + UJ <= k; j += UJ) {
         float4 u4[UJ], v4[UJ];
 #pragma unroll
         for (int q = 0; q < UJ; ++q) {
-          u4[q] = ld_hist<LD>(reinterpret_cast<const float4*>(Ub + (long long)(j + q) * d + i));
-          v4[q] = ld_hist<LD>(reinterpret_cast<const float4*>(Vb + (long long)(j + q) * d + i));
+          u4[q] = __ldg(reinterpret_cast<const float4*>(Ub + (long long)(j + q) * d + i));
+          v4[q] = __ldg(reinterpret_cast<const float4*>(Vb + (long long)(j + q) * d + i));
         }
 #pragma unroll
         for (int q = 0; q < UJ; ++q) {
@@ -364,8 +359,8 @@ k_update(float* __restrict__ x_old, const float* __restrict__ g_old, const float
     for (; j < k; ++j) {
       float u1[VEC], v1[VEC];
       if (VEC == 4) {
-        const float4 u4 = ld_hist<LD>(reinterpret_cast<const float4*>(Ub + (long long)j * d + i));
-        const float4 v4 = ld_hist<LD>(reinterpret_cast<const float4*>(Vb + (long long)j * d + i));
+        const float4 u4 = __ldg(reinterpret_cast<const float4*>(Ub + (long long)j * d + i));
+        const float4 v4 = __ldg(reinterpret_cast<const float4*>(Vb + (long long)j * d + i));
         u1[0] = u4.x; u1[1 % VEC] = u4.y; u1[2 % VEC] = u4.z; u1[3 % VEC] = u4.w;
         v1[0] = v4.x; v1[1 % VEC] = v4.y; v1[2 % VEC] = v4.z; v1[3 % VEC] = v4.w;
       } else {
@@ -451,561 +446,6 @@ k_update(float* __restrict__ x_old, const float* __restrict__ g_old, const float
     } else {
       uk[i] = u[0];
       x_old[base + i] = xnext[0];
-    }
-  }
-  cluster.sync();  // peers may still be reading part1 through DSMEM
-}
-
-// ------------------------------------------------------------------------------------------
-// rank-1 update, cluster per sample, history read from DRAM ONCE (d % 4 == 0).
-// The coefficient of history row j in phase 2 (a_j, b_j, c_j) depends on row j alone, so the history is
-// walked in chunks of G rows: dots of the chunk (first read: DRAM) -> cluster exchange -> accumulation of
-// the chunk into vT, w, S (second read: the rows a CTA touched a few microseconds ago, still in L2 as long
-// as `resident CTAs x 2 G SL 4` bytes fit).  k_update<4> does the same arithmetic with G = k; per-row
-// reduction order, order of the accumulation over j and the expressions are unchanged, so the results are
-// bit-identical.  The running sums live in registers (IT float4 groups per thread = SL / 1024).
-// ------------------------------------------------------------------------------------------
-template <int IT>
-__global__ void __launch_bounds__(kThreads)
-k_update_chunked(float* __restrict__ x_old, const float* __restrict__ g_old, const float* __restrict__ xn,
-                 const float* __restrict__ gn, float* __restrict__ Ut, float* __restrict__ Vt,
-                 float* __restrict__ low_x, float* __restrict__ low_g, const impflow_broyden_state* st, long long d,
-                 int T, int SL, int expect_nstep, int G) {
-  const int do_update = st->do_update;
-  const int new_low = st->new_lowest;
-  if (!do_update && !new_low) return;  // uniform over the whole grid
-  if (expect_nstep >= 0 && st->nstep != expect_nstep) return;
-
-  cg::cluster_group cluster = cg::this_cluster();
-  const int C = cluster.num_blocks();
-  const int r = cluster.block_rank();
-  const int b = blockIdx.x / C;
-  const int k = st->nstep - 1;
-
-  extern __shared__ __align__(16) float smem[];
-  float* sdx = smem;
-  float* sdg = sdx + SL;
-  float* sgn = sdg + SL;
-  float* wsum = sgn + SL;                 // [3*T][kWarps]
-  float* part0 = wsum + 3 * T * kWarps;   // [3*T]
-  float* part1 = part0 + 3 * T;           // [2]
-  float* tot = part1 + 2;                 // [3*T + 2]
-
-  const long long base = (long long)b * d + (long long)r * SL;
-  long long rem = d - (long long)r * SL;
-  const int len = rem <= 0 ? 0 : (rem < SL ? (int)rem : SL);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-
-  // ---- phase 0 ----
-#pragma unroll
-  for (int it = 0; it < IT; ++it) {
-    const int i = tid * 4 + it * kThreads * 4;
-    if (i < len) {
-      const float4 xo = *reinterpret_cast<const float4*>(x_old + base + i);
-      const float4 xv = *reinterpret_cast<const float4*>(xn + base + i);
-      const float4 go = *reinterpret_cast<const float4*>(g_old + base + i);
-      const float4 gv = *reinterpret_cast<const float4*>(gn + base + i);
-      *reinterpret_cast<float4*>(sdx + i) = make_float4(xv.x - xo.x, xv.y - xo.y, xv.z - xo.z, xv.w - xo.w);
-      *reinterpret_cast<float4*>(sdg + i) = make_float4(gv.x - go.x, gv.y - go.y, gv.z - go.z, gv.w - go.w);
-      *reinterpret_cast<float4*>(sgn + i) = gv;
-      if (new_low) {
-        *reinterpret_cast<float4*>(low_x + base + i) = xv;
-        *reinterpret_cast<float4*>(low_g + base + i) = gv;
-      }
-    }
-  }
-  if (!do_update) return;  // uniform
-  __syncthreads();
-
-  const float* Ub = Ut + (long long)b * T * d + (long long)r * SL;
-  const float* Vb = Vt + (long long)b * T * d + (long long)r * SL;
-
-  float vT[IT][4], w[IT][4], S[IT][4];
-#pragma unroll
-  for (int it = 0; it < IT; ++it) {
-    const int i = tid * 4 + it * kThreads * 4;
-#pragma unroll
-    for (int e = 0; e < 4; ++e) {
-      vT[it][e] = (i < len) ? -sdx[i + e] : 0.f;
-      w[it][e] = (i < len) ? -sdg[i + e] : 0.f;
-      S[it][e] = 0.f;
-    }
-  }
-
-  for (int j0 = 0; j0 < k; j0 += G) {
-    const int j1 = (j0 + G < k) ? j0 + G : k;
-    // ---- phase 1 of the chunk: a_j = dx.U_j, b_j = V_j.dg, c_j = V_j.gn (:108,:119) ----
-    for (int j = j0; j < j1; ++j) {
-      const float* uj = Ub + (long long)j * d;
-      const float* vj = Vb + (long long)j * d;
-      float4 u4[IT], v4[IT];
-#pragma unroll
-      for (int it = 0; it < IT; ++it) {
-        const int i = tid * 4 + it * kThreads * 4;
-        if (i < len) {
-          u4[it] = __ldg(reinterpret_cast<const float4*>(uj + i));
-          v4[it] = __ldg(reinterpret_cast<const float4*>(vj + i));
-        }
-      }
-      float a = 0.f, bb = 0.f, c = 0.f;
-#pragma unroll
-      for (int it = 0; it < IT; ++it) {
-        const int i = tid * 4 + it * kThreads * 4;
-        if (i < len) {
-          const float4 dx = *reinterpret_cast<const float4*>(sdx + i);
-          const float4 dg = *reinterpret_cast<const float4*>(sdg + i);
-          const float4 gg = *reinterpret_cast<const float4*>(sgn + i);
-          a += dx.x * u4[it].x + dx.y * u4[it].y + dx.z * u4[it].z + dx.w * u4[it].w;
-          bb += v4[it].x * dg.x + v4[it].y * dg.y + v4[it].z * dg.z + v4[it].w * dg.w;
-          c += v4[it].x * gg.x + v4[it].y * gg.y + v4[it].z * gg.z + v4[it].w * gg.w;
-        }
-      }
-      a = warp_sum(a);
-      bb = warp_sum(bb);
-      c = warp_sum(c);
-      if (lane == 0) {
-        wsum[(3 * j + 0) * kWarps + warp] = a;
-        wsum[(3 * j + 1) * kWarps + warp] = bb;
-        wsum[(3 * j + 2) * kWarps + warp] = c;
-      }
-    }
-    __syncthreads();
-    for (int t = 3 * j0 + tid; t < 3 * j1; t += kThreads) {
-      float s = 0.f;
-      for (int q = 0; q < kWarps; ++q) s += wsum[t * kWarps + q];
-      part0[t] = s;
-    }
-    cluster.sync();      // slots 3*j0 .. 3*j1 are written once per launch: no second barrier per chunk
-    for (int t = 3 * j0 + tid; t < 3 * j1; t += kThreads) {
-      float s = 0.f;
-      for (int q = 0; q < C; ++q) s += cluster.map_shared_rank(part0, q)[t];
-      tot[t] = s;
-    }
-    __syncthreads();
-    // ---- phase 2 of the chunk: vT += a_j V_j, w += b_j U_j, S += c_j U_j (rows re-read from L2) ----
-    for (int j = j0; j < j1; ++j) {
-      const float* uj = Ub + (long long)j * d;
-      const float* vj = Vb + (long long)j * d;
-      const float aj = tot[3 * j + 0], bj = tot[3 * j + 1], cj = tot[3 * j + 2];
-      float4 u4[IT], v4[IT];
-#pragma unroll
-      for (int it = 0; it < IT; ++it) {
-        const int i = tid * 4 + it * kThreads * 4;
-        if (i < len) {
-          u4[it] = __ldg(reinterpret_cast<const float4*>(uj + i));
-          v4[it] = __ldg(reinterpret_cast<const float4*>(vj + i));
-        }
-      }
-#pragma unroll
-      for (int it = 0; it < IT; ++it) {
-        const int i = tid * 4 + it * kThreads * 4;
-        if (i < len) {
-          const float u1[4] = {u4[it].x, u4[it].y, u4[it].z, u4[it].w};
-          const float v1[4] = {v4[it].x, v4[it].y, v4[it].z, v4[it].w};
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            vT[it][e] += aj * v1[e];
-            w[it][e] += bj * u1[e];
-            S[it][e] += cj * u1[e];
-          }
-        }
-      }
-    }
-  }
-
-  // ---- den = vT.dg, c_k = vT_scrubbed.gn; numerator of u and S into smem; store vT (:176-179) ----
-  float den = 0.f, ck = 0.f;
-  float* vk = Vt + (long long)b * T * d + (long long)k * d + (long long)r * SL;
-#pragma unroll
-  for (int it = 0; it < IT; ++it) {
-    const int i = tid * 4 + it * kThreads * 4;
-    if (i < len) {
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        const float dx = sdx[i + e], dg = sdg[i + e], gg = sgn[i + e];
-        den += vT[it][e] * dg;                                         // unscrubbed vT in the denominator (:176)
-        vT[it][e] = (vT[it][e] != vT[it][e]) ? 0.f : vT[it][e];        // :177
-        ck += vT[it][e] * gg;
-        sdx[i + e] = dx - w[it][e];                                    // numerator of u
-        sdg[i + e] = S[it][e];
-      }
-      *reinterpret_cast<float4*>(vk + i) = make_float4(vT[it][0], vT[it][1], vT[it][2], vT[it][3]);  // :179
-    }
-  }
-  den = warp_sum(den);
-  ck = warp_sum(ck);
-  if (lane == 0) {
-    wsum[warp] = den;
-    wsum[kWarps + warp] = ck;
-  }
-  __syncthreads();
-  if (tid < 2) {
-    float s = 0.f;
-    for (int q = 0; q < kWarps; ++q) s += wsum[tid * kWarps + q];
-    part1[tid] = s;
-  }
-  cluster.sync();
-  if (tid < 2) {
-    float s = 0.f;
-    for (int q = 0; q < C; ++q) s += cluster.map_shared_rank(part1, q)[tid];
-    tot[3 * T + tid] = s;
-  }
-  __syncthreads();
-  const float den_t = tot[3 * T + 0], ck_t = tot[3 * T + 1];
-
-  // ---- phase 3: u (scrub), next direction and next iterate (:176-181, :90) ----
-  float* uk = Ut + (long long)b * T * d + (long long)k * d + (long long)r * SL;
-#pragma unroll
-  for (int it = 0; it < IT; ++it) {
-    const int i = tid * 4 + it * kThreads * 4;
-    if (i < len) {
-      const float4 x4 = *reinterpret_cast<const float4*>(xn + base + i);
-      const float xv[4] = {x4.x, x4.y, x4.z, x4.w};
-      float u[4], xnext[4];
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        float q = sdx[i + e] / den_t;
-        q = (q != q) ? 0.f : q;                        // :178
-        u[e] = q;
-        const float upd = -((-sgn[i + e]) + (sdg[i + e] + q * ck_t));  // -matvec(U[:nstep], V[:nstep], gx) :181
-        xnext[e] = xv[e] + upd;
-      }
-      *reinterpret_cast<float4*>(uk + i) = make_float4(u[0], u[1], u[2], u[3]);   // :180
-      *reinterpret_cast<float4*>(x_old + base + i) = make_float4(xnext[0], xnext[1], xnext[2], xnext[3]);
-    }
-  }
-  cluster.sync();  // peers may still be reading part1 through DSMEM
-}
-
-// ------------------------------------------------------------------------------------------
-// rank-1 update for histories that do not fit in L2 (classifier shapes: B = 128, d = 65536, 2 GB): every history
-// row crosses the SM boundary ONCE.  Cluster per sample, slices of <= 4096 floats.  A producer warp streams the
-// (U_j, V_j) slices through a ring of kStreamStages shared-memory stages with 1-D bulk copies (cp.async.bulk,
-// completion counted on an mbarrier); the 8 compute warps take the three dots of row j from shared memory, PUSH the
-// block sums into every peer's shared memory (st.shared::cluster + remote mbarrier arrive: no blocking cluster
-// barrier, several rows in flight) and, kStreamAhead rows later, accumulate row j into vT, w, S from the SAME stage.
-// Reduction order per row: thread partial (ascending i) -> warp tree -> warps ascending -> ranks ascending, as in
-// k_update<4>; only the slice length differs (so results agree to round-off, not bit for bit).
-// dynamic smem: sdx[SL] sdg[SL] | ring[kStreamStages][2][SL] | parts[T][3][C] | wsum[3][8] bsum[4] part1[2] tot1[2]
-//               | full[kStreamStages] empty[kStreamStages] xbar[T]
-// ------------------------------------------------------------------------------------------
-constexpr int kStreamStages = 5;
-constexpr int kStreamAhead = 2;
-constexpr int kStreamIT = 4;            // float4 groups per thread: slices of <= 4096 floats
-constexpr int kStreamThreads = kThreads + 32;
-
-__device__ __forceinline__ uint32_t s_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void sb_init(uint64_t* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(s_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void sb_expect_tx(uint64_t* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(s_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void sb_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(s_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void sb_wait(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "SB_WAIT:\n\t"
-      "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra.uni SB_DONE;\n\t"
-      "bra.uni SB_WAIT;\n\t"
-      "SB_DONE:\n\t"
-      "}\n" ::"r"(s_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-// wait for arrivals that peers made with release.cluster (their st.shared::cluster stores become visible)
-__device__ __forceinline__ void sb_wait_cluster(uint64_t* bar, uint32_t parity) {
-  asm volatile(
-      "{\n\t"
-      ".reg .pred p;\n\t"
-      "SBC_WAIT:\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n\t"
-      "@p bra.uni SBC_DONE;\n\t"
-      "bra.uni SBC_WAIT;\n\t"
-      "SBC_DONE:\n\t"
-      "}\n" ::"r"(s_u32(bar)),
-      "r"(parity)
-      : "memory");
-}
-__device__ __forceinline__ uint32_t map_to_rank(const void* p, uint32_t rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(s_u32(p)), "r"(rank));
-  return r;
-}
-__device__ __forceinline__ void st_remote(uint32_t addr, float v) {
-  asm volatile("st.shared::cluster.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
-}
-__device__ __forceinline__ void arrive_remote(uint32_t bar_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(bar_addr) : "memory");
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-                   s_u32(dst)),
-               "l"(src), "r"(bytes), "r"(s_u32(bar))
-               : "memory");
-}
-__device__ __forceinline__ void compute_bar() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
-
-__global__ void __launch_bounds__(kStreamThreads, 1)
-k_update_stream(float* __restrict__ x_old, const float* __restrict__ g_old, const float* __restrict__ xn,
-                const float* __restrict__ gn, float* __restrict__ Ut, float* __restrict__ Vt,
-                float* __restrict__ low_x, float* __restrict__ low_g, const impflow_broyden_state* st, long long d,
-                int T, int SL, int expect_nstep) {
-  constexpr int IT = kStreamIT;
-  const int do_update = st->do_update;
-  const int new_low = st->new_lowest;
-  if (!do_update && !new_low) return;  // uniform over the whole grid
-  if (expect_nstep >= 0 && st->nstep != expect_nstep) return;
-
-  cg::cluster_group cluster = cg::this_cluster();
-  const int C = cluster.num_blocks();
-  const int r = cluster.block_rank();
-  const int b = blockIdx.x / C;
-  const int k = st->nstep - 1;
-
-  extern __shared__ __align__(16) float smem[];
-  float* sdx = smem;
-  float* sdg = sdx + SL;
-  float* ring = sdg + SL;                                   // [stage][U | V][SL]
-  float* parts = ring + (size_t)kStreamStages * 2 * SL;     // [T][3][C]
-  float* wsum = parts + (size_t)T * 3 * C;                  // [3][kWarps]
-  float* bsum = wsum + 3 * kWarps;                          // [4]
-  float* part1 = bsum + 4;                                  // [2]
-  float* tot1 = part1 + 2;                                  // [2]
-  uint64_t* full = reinterpret_cast<uint64_t*>(tot1 + 2 + (((size_t)T * 3 * C) & 1));   // 8-byte aligned
-  uint64_t* empty = full + kStreamStages;
-  uint64_t* xbar = empty + kStreamStages;                   // [T]
-
-  const long long base = (long long)b * d + (long long)r * SL;
-  long long rem = d - (long long)r * SL;
-  const int len = rem <= 0 ? 0 : (rem < SL ? (int)rem : SL);
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const bool compute = tid < kThreads;
-
-  // ---- phase 0: deltas into smem (g_new stays in registers), best-iterate copy ----
-  float4 gg[IT];
-  if (compute) {
-    float4 xo[IT], xv[IT], go[IT];
-#pragma unroll
-    for (int it = 0; it < IT; ++it) {
-      const int i = tid * 4 + it * kThreads * 4;
-      if (i < len) {
-        xo[it] = *reinterpret_cast<const float4*>(x_old + base + i);
-        xv[it] = *reinterpret_cast<const float4*>(xn + base + i);
-        go[it] = *reinterpret_cast<const float4*>(g_old + base + i);
-        gg[it] = *reinterpret_cast<const float4*>(gn + base + i);
-      }
-    }
-#pragma unroll
-    for (int it = 0; it < IT; ++it) {
-      const int i = tid * 4 + it * kThreads * 4;
-      if (i < len) {
-        *reinterpret_cast<float4*>(sdx + i) =
-            make_float4(xv[it].x - xo[it].x, xv[it].y - xo[it].y, xv[it].z - xo[it].z, xv[it].w - xo[it].w);
-        *reinterpret_cast<float4*>(sdg + i) =
-            make_float4(gg[it].x - go[it].x, gg[it].y - go[it].y, gg[it].z - go[it].z, gg[it].w - go[it].w);
-        if (new_low) {
-          *reinterpret_cast<float4*>(low_x + base + i) = xv[it];
-          *reinterpret_cast<float4*>(low_g + base + i) = gg[it];
-        }
-      } else {
-        gg[it] = make_float4(0.f, 0.f, 0.f, 0.f);
-      }
-    }
-  }
-  if (!do_update) return;  // uniform
-  if (tid == 0) {
-    for (int s = 0; s < kStreamStages; ++s) {
-      sb_init(full + s, 1);
-      sb_init(empty + s, kWarps);
-    }
-    for (int j = 0; j < T; ++j) sb_init(xbar + j, C);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  __syncthreads();
-  cluster.sync();       // every peer's barriers exist before the first remote arrive
-
-  const float* Ub = Ut + (long long)b * T * d + (long long)r * SL;
-  const float* Vb = Vt + (long long)b * T * d + (long long)r * SL;
-  const uint32_t row_bytes = (uint32_t)len * 4u;
-
-  float vT[IT][4], w[IT][4], S[IT][4];
-  if (!compute) {
-    // ---- producer warp: one lane streams the history slices through the ring ----
-    if (lane == 0) {
-      for (int j = 0; j < k; ++j) {
-        const int s = j % kStreamStages;
-        if (j >= kStreamStages) sb_wait(empty + s, ((j / kStreamStages) - 1) & 1);
-        sb_expect_tx(full + s, 2 * row_bytes);
-        if (row_bytes) {
-          bulk_g2s(ring + (size_t)s * 2 * SL, Ub + (long long)j * d, row_bytes, full + s);
-          bulk_g2s(ring + (size_t)s * 2 * SL + SL, Vb + (long long)j * d, row_bytes, full + s);
-        }
-      }
-    }
-  } else {
-#pragma unroll
-    for (int it = 0; it < IT; ++it) {
-      const int i = tid * 4 + it * kThreads * 4;
-#pragma unroll
-      for (int e = 0; e < 4; ++e) {
-        vT[it][e] = (i < len) ? -sdx[i + e] : 0.f;
-        w[it][e] = (i < len) ? -sdg[i + e] : 0.f;
-        S[it][e] = 0.f;
-      }
-    }
-    // dots of row j from its stage; block sums pushed to every peer (a_j = dx.U_j, b_j = V_j.dg, c_j = V_j.gn)
-    auto dots_push = [&](int j) {
-      const int s = j % kStreamStages;
-      sb_wait(full + s, (j / kStreamStages) & 1);
-      const float* us = ring + (size_t)s * 2 * SL;
-      const float* vs = us + SL;
-      float a = 0.f, bb = 0.f, c = 0.f;
-#pragma unroll
-      for (int it = 0; it < IT; ++it) {
-        const int i = tid * 4 + it * kThreads * 4;
-        if (i < len) {
-          const float4 u4 = *reinterpret_cast<const float4*>(us + i);
-          const float4 v4 = *reinterpret_cast<const float4*>(vs + i);
-          const float4 dx = *reinterpret_cast<const float4*>(sdx + i);
-          const float4 dg = *reinterpret_cast<const float4*>(sdg + i);
-          a += dx.x * u4.x + dx.y * u4.y + dx.z * u4.z + dx.w * u4.w;
-          bb += v4.x * dg.x + v4.y * dg.y + v4.z * dg.z + v4.w * dg.w;
-          c += v4.x * gg[it].x + v4.y * gg[it].y + v4.z * gg[it].z + v4.w * gg[it].w;
-        }
-      }
-      a = warp_sum(a);
-      bb = warp_sum(bb);
-      c = warp_sum(c);
-      compute_bar();      // the previous row's wsum / bsum have been consumed
-      if (lane == 0) {
-        wsum[0 * kWarps + warp] = a;
-        wsum[1 * kWarps + warp] = bb;
-        wsum[2 * kWarps + warp] = c;
-      }
-      compute_bar();
-      if (warp == 0) {
-        if (lane < 3) {
-          float t = 0.f;
-          for (int q = 0; q < kWarps; ++q) t += wsum[lane * kWarps + q];
-          bsum[lane] = t;
-        }
-        __syncwarp();
-        if (lane < C) {
-          float* slot = parts + ((size_t)j * 3) * C + r;      // parts[j][t][source rank]
-          st_remote(map_to_rank(slot, lane), bsum[0]);
-          st_remote(map_to_rank(slot + C, lane), bsum[1]);
-          st_remote(map_to_rank(slot + 2 * C, lane), bsum[2]);
-          arrive_remote(map_to_rank(xbar + j, lane));
-        }
-      }
-    };
-    const int ahead = k < kStreamAhead ? k : kStreamAhead;
-    for (int j = 0; j < ahead; ++j) dots_push(j);
-    for (int j = 0; j < k; ++j) {
-      if (j + kStreamAhead < k) dots_push(j + kStreamAhead);
-      sb_wait_cluster(xbar + j, 0);
-      float aj = 0.f, bj = 0.f, cj = 0.f;
-      const float* pj = parts + ((size_t)j * 3) * C;
-      for (int q = 0; q < C; ++q) {
-        aj += pj[q];
-        bj += pj[C + q];
-        cj += pj[2 * C + q];
-      }
-      const int s = j % kStreamStages;
-      const float* us = ring + (size_t)s * 2 * SL;
-      const float* vs = us + SL;
-#pragma unroll
-      for (int it = 0; it < IT; ++it) {
-        const int i = tid * 4 + it * kThreads * 4;
-        if (i < len) {
-          const float4 u4 = *reinterpret_cast<const float4*>(us + i);
-          const float4 v4 = *reinterpret_cast<const float4*>(vs + i);
-          const float u1[4] = {u4.x, u4.y, u4.z, u4.w};
-          const float v1[4] = {v4.x, v4.y, v4.z, v4.w};
-#pragma unroll
-          for (int e = 0; e < 4; ++e) {
-            vT[it][e] += aj * v1[e];
-            w[it][e] += bj * u1[e];
-            S[it][e] += cj * u1[e];
-          }
-        }
-      }
-      __syncwarp();
-      if (lane == 0) sb_arrive(empty + s);      // this warp is done with the stage
-    }
-  }
-
-  // ---- den = vT.dg, c_k = vT_scrubbed.gn; numerator of u and S into smem; store vT (:176-179) ----
-  float* vk = Vt + (long long)b * T * d + (long long)k * d + (long long)r * SL;
-  if (compute) {
-    float den = 0.f, ck = 0.f;
-#pragma unroll
-    for (int it = 0; it < IT; ++it) {
-      const int i = tid * 4 + it * kThreads * 4;
-      if (i < len) {
-        const float g4[4] = {gg[it].x, gg[it].y, gg[it].z, gg[it].w};
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          const float dx = sdx[i + e], dg = sdg[i + e];
-          den += vT[it][e] * dg;                                         // unscrubbed vT in the denominator (:176)
-          vT[it][e] = (vT[it][e] != vT[it][e]) ? 0.f : vT[it][e];        // :177
-          ck += vT[it][e] * g4[e];
-          sdx[i + e] = dx - w[it][e];                                    // numerator of u
-          sdg[i + e] = S[it][e];
-        }
-        *reinterpret_cast<float4*>(vk + i) = make_float4(vT[it][0], vT[it][1], vT[it][2], vT[it][3]);  // :179
-      }
-    }
-    den = warp_sum(den);
-    ck = warp_sum(ck);
-    compute_bar();
-    if (lane == 0) {
-      wsum[warp] = den;
-      wsum[kWarps + warp] = ck;
-    }
-    compute_bar();
-    if (tid < 2) {
-      float t = 0.f;
-      for (int q = 0; q < kWarps; ++q) t += wsum[tid * kWarps + q];
-      part1[tid] = t;
-    }
-  }
-  cluster.sync();
-  if (tid < 2) {
-    float t = 0.f;
-    for (int q = 0; q < C; ++q) t += cluster.map_shared_rank(part1, q)[tid];
-    tot1[tid] = t;
-  }
-  __syncthreads();
-  const float den_t = tot1[0], ck_t = tot1[1];
-
-  // ---- phase 3: u (scrub), next direction and next iterate (:176-181, :90) ----
-  float* uk = Ut + (long long)b * T * d + (long long)k * d + (long long)r * SL;
-  if (compute) {
-#pragma unroll
-    for (int it = 0; it < IT; ++it) {
-      const int i = tid * 4 + it * kThreads * 4;
-      if (i < len) {
-        const float4 x4 = *reinterpret_cast<const float4*>(xn + base + i);
-        const float xv[4] = {x4.x, x4.y, x4.z, x4.w};
-        const float g4[4] = {gg[it].x, gg[it].y, gg[it].z, gg[it].w};
-        float u[4], xnext[4];
-#pragma unroll
-        for (int e = 0; e < 4; ++e) {
-          float q = sdx[i + e] / den_t;
-          q = (q != q) ? 0.f : q;                        // :178
-          u[e] = q;
-          const float upd = -((-g4[e]) + (sdg[i + e] + q * ck_t));  // -matvec(U[:nstep], V[:nstep], gx) :181
-          xnext[e] = xv[e] + upd;
-        }
-        *reinterpret_cast<float4*>(uk + i) = make_float4(u[0], u[1], u[2], u[3]);   // :180
-        *reinterpret_cast<float4*>(x_old + base + i) = make_float4(xnext[0], xnext[1], xnext[2], xnext[3]);
-      }
     }
   }
   cluster.sync();  // peers may still be reading part1 through DSMEM
@@ -1097,17 +537,6 @@ k_update_small(float* __restrict__ x_old, const float* __restrict__ g_old, const
   }
 }
 
-// update kernel selection (impflow_broyden_set_chunk), all measured at B = 128, d = 65536 (2 GB of history), 15
-// iterations, algorithmic bytes / time against 6543 GB/s (scripts/update_bench.py, profiles/r02_update_bench.txt):
-//   -1 / 0  k_update<4, 256>   two passes over the history, 16 loads per thread in flight        0.41  (default)
-//   -3      k_update<4, 512>   the same with 16 warps per CTA                                     0.42
-//   -2      k_update_stream    every row crosses the SM boundary once (bulk-copy ring, pushes)    0.28
-//   n > 0   k_update_chunked   two passes in chunks of n rows, second pass from L2                0.31
-// ncu (profiles/r02_ncu_k_update.txt): none of them is DRAM-bound (47 % DRAM throughput at rank 8); the two-pass
-// kernel is issue / latency bound at 14.5 resident warps per SM (96 KB of shared memory per CTA), the read-once
-// variants pay more for their per-row exchange than they save in traffic.
-static int g_update_chunk = -1;
-
 static int pick_splits(int B, long long d) {
   int S = 1;
   while ((long long)B * S < 592 && d / (S * 2) >= 2048 && S < 64) S *= 2;
@@ -1129,12 +558,6 @@ static void pick_cluster(int B, long long d, int* C_out, int* SL_out) {
 
 using namespace impflow;
 
-extern "C" int impflow_broyden_set_chunk(int rows) {
-  const int was = g_update_chunk;
-  g_update_chunk = rows;
-  return was;
-}
-
 extern "C" size_t impflow_broyden_state_bytes(void) { return sizeof(impflow_broyden_state); }
 
 extern "C" size_t impflow_broyden_workspace_floats(int B, long long d, int threshold) {
@@ -1145,56 +568,6 @@ extern "C" size_t impflow_broyden_workspace_floats(int B, long long d, int thres
 static int launch_norm(const float* g, float* partial, float* sample_sq, float* low_sq,
                        impflow_broyden_state* state, int B, long long d, int init, int gated,
                        BroydenProgress* progress, cudaStream_t s);
-
-// history-streaming update kernel: 0 = launched, -1 = error, 1 = the cluster shape cannot be scheduled here
-static int launch_update_stream(float* x_old, const float* g_old, const float* xn, const float* gn, float* Ut,
-                                float* Vt, float* low_x, float* low_g, impflow_broyden_state* state, int B,
-                                long long d, int threshold, int expect_nstep, cudaStream_t s) {
-  int C = 1;
-  while (C < 16 && (d + C - 1) / C > 1024 * kStreamIT) C *= 2;
-  long long sl = (d + C - 1) / C;
-  sl = (sl + 3) / 4 * 4;
-  const int SL = (int)sl;
-  const size_t floats = (size_t)2 * SL + (size_t)kStreamStages * 2 * SL + (size_t)threshold * 3 * C + 3 * kWarps + 4 +
-                        2 + 2 + 2;
-  const size_t smem = floats * sizeof(float) + sizeof(uint64_t) * (2 * kStreamStages + threshold) + 16;
-  static int configured = 0;      // 0 unknown, 1 ok, -1 unsupported
-  if (configured == 0) {
-    bool ok = cudaFuncSetAttribute(k_update_stream, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024) ==
-              cudaSuccess;
-    ok = ok && cudaFuncSetAttribute(k_update_stream, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess;
-    configured = ok ? 1 : -1;
-    if (!ok) cudaGetLastError();
-  }
-  if (configured < 0 || smem > 227 * 1024) return 1;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)(B * C));
-  cfg.blockDim = dim3(kStreamThreads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = C;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  static int placed[17] = {0};    // per cluster size: 0 unknown, 1 schedulable, -1 not
-  if (placed[C] == 0) {
-    int n = 0;
-    placed[C] = (cudaOccupancyMaxActiveClusters(&n, k_update_stream, &cfg) == cudaSuccess && n > 0) ? 1 : -1;
-    if (placed[C] < 0) cudaGetLastError();
-  }
-  if (placed[C] < 0) return 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, k_update_stream, x_old, g_old, xn, gn, Ut, Vt, low_x, low_g,
-                                     (const impflow_broyden_state*)state, d, threshold, SL, expect_nstep);
-  if (e != cudaSuccess) {
-    set_error("broyden_step: stream-kernel cluster launch failed: %s", cudaGetErrorString(e));
-    return -1;
-  }
-  return check_launch("k_update_stream");
-}
 
 extern "C" int impflow_broyden_begin(const float* x0, const float* g0, float* xn, float* low_x, float* low_g,
                                      float* sample_sq, float* low_sq, float* partial,
@@ -1250,49 +623,26 @@ int impflow::broyden_step_ex(float* x_old, const float* g_old, const float* xn, 
     return check_launch("k_update_small");
   }
   IMPFLOW_REQUIRE(d <= 8LL * 8192, "broyden: d=%lld exceeds the cluster kernel limit 65536", d);
-  if ((d % 4) == 0 && d >= 2048 && g_update_chunk == -2) {
-    const int rc = launch_update_stream(x_old, g_old, xn, gn, Ut, Vt, low_x, low_g, state, B, d, threshold,
-                                        expect_nstep, s);
-    if (rc <= 0) return rc;     // > 0: this device cannot place the cluster; fall through to the two-pass kernel
-  }
   int C, SL;
   pick_cluster(B, d, &C, &SL);
+  // wsum is sized for 16 warps although k_update runs 8: the bytes bound how many CTAs share an SM, so shrinking
+  // them is a performance change of its own
   const size_t smem = sizeof(float) * ((size_t)3 * SL + (size_t)3 * threshold * 16 + 3 * threshold + 2 +
-                                       3 * threshold + 2 + 8);      // wsum sized for the 16-warp variant
-  const bool vec = (d % 4 == 0);
-  // k_update_chunked (history walked in chunks of rows whose second pass hits L2) only on request: measured not
-  // faster than the two-pass kernel, both are bound by load latency rather than by DRAM bytes
-  const int G = (vec && g_update_chunk > 0) ? g_update_chunk : 0;
-  // two-pass kernel variants (impflow_broyden_set_chunk codes -3 / -4 / -5 for A/B): 512 threads per CTA double the
-  // loads in flight per SM (the kernel is latency bound at 16 warps per SM); L1-bypassing history loads
-  int nt = 256;
+                                       3 * threshold + 2 + 8);
+  // The two-pass kernel is kept on purpose: read-once variants (history streamed through a bulk-copy ring, or walked
+  // in L2-sized row chunks) were measured slower, 512-thread / L1-bypassing ones within a few per cent and not adopted
+  // (profiles/r02_update_bench.txt; their source is in commits de6f192 and 74f3be3).
   void (*kern)(float*, const float*, const float*, const float*, float*, float*, float*, float*,
-               const impflow_broyden_state*, long long, int, int, int) = vec ? k_update<4, 256, 0> : k_update<1, 256, 0>;
-  size_t smem_pad = 0;
-  if (vec && SL >= 2048 && (g_update_chunk == -3 || g_update_chunk == -4 || g_update_chunk == -6)) {
-    nt = 512;
-    kern = g_update_chunk == -4 ? k_update<4, 512, 1> : k_update<4, 512, 0>;
-    if (g_update_chunk == -6) smem_pad = 120 * 1024;      // one CTA per SM: half the history in flight (fits L2)
-  } else if (vec && g_update_chunk == -5) {
-    kern = k_update<4, 256, 1>;
-  }
-  const size_t smem_launch = smem > smem_pad ? smem : smem_pad;
-  void (*kern_c)(float*, const float*, const float*, const float*, float*, float*, float*, float*,
-                 const impflow_broyden_state*, long long, int, int, int, int) = nullptr;
-  if (G > 0) {
-    kern_c = SL <= 1024 ? k_update_chunked<1> : SL <= 2048 ? k_update_chunked<2> : SL <= 4096 ? k_update_chunked<4>
-                                                                                             : k_update_chunked<8>;
-  }
-  if ((kern_c ? cudaFuncSetAttribute(kern_c, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_launch)
-              : cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_launch)) != cudaSuccess) {
+               const impflow_broyden_state*, long long, int, int, int) = d % 4 == 0 ? k_update<4> : k_update<1>;
+  if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
     set_error("broyden_step: cannot set %zu bytes of dynamic shared memory", smem);
     return -1;
   }
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3((unsigned)(B * C));
-  cfg.blockDim = dim3(kern_c ? kThreads : nt);
-  cfg.dynamicSmemBytes = smem_launch;
+  cfg.blockDim = dim3(kThreads);
+  cfg.dynamicSmemBytes = smem;
   cfg.stream = s;
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension;
@@ -1301,10 +651,8 @@ int impflow::broyden_step_ex(float* x_old, const float* g_old, const float* xn, 
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  cudaError_t e = kern_c ? cudaLaunchKernelEx(&cfg, kern_c, x_old, g_old, xn, gn, Ut, Vt, low_x, low_g,
-                                              (const impflow_broyden_state*)state, d, threshold, SL, expect_nstep, G)
-                         : cudaLaunchKernelEx(&cfg, kern, x_old, g_old, xn, gn, Ut, Vt, low_x, low_g,
-                                              (const impflow_broyden_state*)state, d, threshold, SL, expect_nstep);
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, x_old, g_old, xn, gn, Ut, Vt, low_x, low_g,
+                                     (const impflow_broyden_state*)state, d, threshold, SL, expect_nstep);
   if (e != cudaSuccess) {
     set_error("broyden_step: cluster launch failed: %s", cudaGetErrorString(e));
     return -1;

@@ -18,9 +18,8 @@
 //   phase B  (tensor pipe): for every pass of <= 128 tap columns: ACC3 = A2 W3[pass, q]^T (A from tensor memory,
 //                           W3 chunks through the same ring), read back by the 16 warps into the partial Y_q
 // Operand traffic: a single CTA pulls 64 KB (A1 chunk + W2 chunk) through L2 per 768 tensor-pipe cycles, twice
-// what the L2 delivers to every SM at once — so when C = 512 the four quarter-CTAs of one row tile form a CLUSTER:
-// each of them loads a quarter of the shared A1 chunk and TMA-multicasts it to all four (40 KB per CTA and chunk
-// instead of 64), the ring's empty barriers collect the MMA commits of all four CTAs (tcgen05.commit multicast).
+// what the L2 delivers to every SM at once.  Sharing the A1 chunk among the four quarter-CTAs of a row tile by TMA
+// multicast was measured slower (91 vs 123 TFLOP/s, DESIGN.md §4) and removed.
 // The Q = C/128 partials are summed in fixed order by the col2im kernel that follows (k_conv3_out), so the result
 // does not depend on the order in which the quarters finish.  Everything is fp32-accurate 3xTF32.
 #include "tile_common.cuh"
@@ -61,7 +60,7 @@ struct Chain23Args {
 // and 3 split every landed chunk into tf32 hi / lo planes in shared memory (round-to-nearest hi in place, lo = a - hi
 // beside it) before the MMAs read it.  A CTA then pulls 48 KB instead of 64 KB through L2 per K chunk - the stream that
 // bounds this kernel - and the layer-1 GEMM's epilogue writes 4 instead of 8 bytes per element.
-template <int ACT, bool MC, bool A32>
+template <int ACT, bool A32>
 __global__ void __launch_bounds__(C23_THREADS, 1)
 k_chain23(const __grid_constant__ CUtensorMap mapAhi, const __grid_constant__ CUtensorMap mapAlo,
           const __grid_constant__ CUtensorMap mapW2hi, const __grid_constant__ CUtensorMap mapW2lo,
@@ -101,7 +100,7 @@ k_chain23(const __grid_constant__ CUtensorMap mapAhi, const __grid_constant__ CU
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < C23_NS; ++s) {
       mbar_init(&full[s], 1);
-      mbar_init(&empty[s], MC ? 4 : 1);      // MC: the MMA commits of all four CTAs of the cluster
+      mbar_init(&empty[s], 1);
       mbar_init(&ready[s], 2);               // warps 2 and 3
     }
     mbar_init(acc2_full, 1);
@@ -120,10 +119,8 @@ k_chain23(const __grid_constant__ CUtensorMap mapAhi, const __grid_constant__ CU
   }
   tc_fence_before();
   __syncthreads();
-  if (MC) cluster_barrier();   // the peers' barriers are initialised before anything signals them
   tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  const uint32_t crank = MC ? cluster_rank() : 0u;
   pdl_wait();        // the set-up above overlapped the predecessor (the layer-1 GEMM); no global memory touched yet
   if (gate_closed(args.gate)) num_items = 0;   // speculative solver iteration after the loop ended (uniform)
 
@@ -141,10 +138,6 @@ k_chain23(const __grid_constant__ CUtensorMap mapAhi, const __grid_constant__ CU
           mbar_expect_tx(&full[st], A32 ? 3 * C23_PLANE : C23_STAGE_BYTES);
           if (A32) {     // one fp32 plane; the lo plane of the stage is produced on chip
             tma_load_2d(&mapAhi, &full[st], sp, kc * TC_BK, m0);
-          } else if (MC) {      // this CTA's 32 rows of the shared A1 chunk, multicast to the four CTAs of the row tile
-            tma_load_2d_mc(&mapAhi, &full[st], sp + crank * 4096, kc * TC_BK, m0 + (int)crank * 32, (uint16_t)0xF);
-            tma_load_2d_mc(&mapAlo, &full[st], sp + C23_PLANE + crank * 4096, kc * TC_BK, m0 + (int)crank * 32,
-                           (uint16_t)0xF);
           } else {
             tma_load_2d(&mapAhi, &full[st], sp, kc * TC_BK, m0);
             tma_load_2d(&mapAlo, &full[st], sp + C23_PLANE, kc * TC_BK, m0);
@@ -197,8 +190,7 @@ k_chain23(const __grid_constant__ CUtensorMap mapAhi, const __grid_constant__ CU
             umma_tf32(t_acc2, dah, dbl, idesc2, 1u);                               // hi * lo
             umma_tf32(t_acc2, dah, dbh, idesc2, 1u);                               // hi * hi
           }
-          if (MC) umma_commit_mc(&empty[st], (uint16_t)0xF);
-          else umma_commit(&empty[st]);
+          umma_commit(&empty[st]);
           if (kc == NC - 1) umma_commit(acc2_full);
         }
         __syncwarp();
@@ -225,8 +217,7 @@ k_chain23(const __grid_constant__ CUtensorMap mapAhi, const __grid_constant__ CU
               umma_tf32_ts(t_acc3, t_a2hi + col, dbl, idesc3, 1u);
               umma_tf32_ts(t_acc3, t_a2hi + col, dbh, idesc3, 1u);
             }
-            if (MC) umma_commit_mc(&empty[st], (uint16_t)0xF);
-            else umma_commit(&empty[st]);
+            umma_commit(&empty[st]);
             if (c2 == NC3 - 1) {
               umma_commit(acc3_full);
               if (j == args.npass - 1) umma_commit(a2_empty);
@@ -349,20 +340,17 @@ k_chain23(const __grid_constant__ CUtensorMap mapAhi, const __grid_constant__ CU
   }
   tc_fence_before();
   __syncthreads();
-  if (MC) cluster_barrier();   // no CTA leaves while a peer may still multicast into it or arrive on its barriers
   if (warp == 2) {
     tc_fence_after();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512u) : "memory");
   }
 }
 
-static int g_chain23_mc = 0;     // cluster-multicast variant (impflow_chain23_set_multicast): measured SLOWER (91 vs 123 TFLOP/s), off
-
-template <int ACT, bool MC, bool A32>
+template <int ACT, bool A32>
 static int launch_chain23(const CUtensorMap* maps, const Chain23Args& a, cudaStream_t s) {
   static bool attr_set = false;
   if (!attr_set) {
-    if (cudaFuncSetAttribute(k_chain23<ACT, MC, A32>, cudaFuncAttributeMaxDynamicSharedMemorySize, C23_SMEM_BYTES) !=
+    if (cudaFuncSetAttribute(k_chain23<ACT, A32>, cudaFuncAttributeMaxDynamicSharedMemorySize, C23_SMEM_BYTES) !=
         cudaSuccess) {
       set_error("chain23_tc: cannot set %d bytes of dynamic shared memory", C23_SMEM_BYTES);
       return -1;
@@ -370,26 +358,17 @@ static int launch_chain23(const CUtensorMap* maps, const Chain23Args& a, cudaStr
     attr_set = true;
   }
   const long long items = ((a.M + TC_BM - 1) / TC_BM) * (a.C / 128);
-  const int grid = (int)(items < 148 ? items : 148);     // 148 = 37 clusters of four; items is a multiple of four
+  const int grid = (int)(items < 148 ? items : 148);     // persistent: at most one CTA per SM
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3(grid);
   cfg.blockDim = dim3(C23_THREADS);
   cfg.dynamicSmemBytes = C23_SMEM_BYTES;
   cfg.stream = s;
-  cudaLaunchAttribute attr[2];
+  cudaLaunchAttribute attr[1];
   cfg.attrs = attr;
-  int na = 0;
-  if (MC) {
-    attr[na].id = cudaLaunchAttributeClusterDimension;
-    attr[na].val.clusterDim.x = 4;
-    attr[na].val.clusterDim.y = 1;
-    attr[na].val.clusterDim.z = 1;
-    ++na;
-  }
-  na += pdl_attr(&attr[na]);
-  cfg.numAttrs = na;
-  const cudaError_t err = cudaLaunchKernelEx(&cfg, k_chain23<ACT, MC, A32>, maps[0], maps[1], maps[2], maps[3], maps[4], maps[5], a);
+  cfg.numAttrs = pdl_attr(&attr[0]);
+  const cudaError_t err = cudaLaunchKernelEx(&cfg, k_chain23<ACT, A32>, maps[0], maps[1], maps[2], maps[3], maps[4], maps[5], a);
   if (err != cudaSuccess) {
     set_error("k_chain23: launch failed: %s", cudaGetErrorString(err));
     return -1;
@@ -402,12 +381,6 @@ static int launch_chain23(const CUtensorMap* maps, const Chain23Args& a, cudaStr
 using namespace impflow;
 
 extern "C" int impflow_chain23_parts(int C) { return C / 128; }
-
-extern "C" int impflow_chain23_set_multicast(int on) {
-  const int prev = g_chain23_mc;
-  g_chain23_mc = on ? 1 : 0;
-  return prev;
-}
 
 extern "C" int impflow_chain23_tc(const float* A_hi, const float* A_lo, long long lda, const float* W2_hi,
                                   const float* W2_lo, const float* W3_hi, const float* W3_lo, const float* bias2,
@@ -430,10 +403,8 @@ extern "C" int impflow_chain23_tc(const float* A_hi, const float* A_lo, long lon
     return -2;
   }
   const bool a32 = A_lo == nullptr;              // one fp32 plane, split on chip
-  const bool mc = !a32 && g_chain23_mc && C == 512;      // four quarter-CTAs per row tile = one cluster
   CUtensorMap maps[6];
-  if (make_map(&maps[0], A_hi, M, C, lda, mc ? 32 : 128) ||
-      make_map(&maps[1], a32 ? A_hi : A_lo, M, C, lda, mc ? 32 : 128) ||
+  if (make_map(&maps[0], A_hi, M, C, lda, 128) || make_map(&maps[1], a32 ? A_hi : A_lo, M, C, lda, 128) ||
       make_map(&maps[2], W2_hi, C, C, C, 128) || make_map(&maps[3], W2_lo, C, C, C, 128) ||
       make_map(&maps[4], W3_hi, N3, C, C, 128) || make_map(&maps[5], W3_lo, N3, C, C, 128))
     return -1;
@@ -448,24 +419,16 @@ extern "C" int impflow_chain23_tc(const float* A_hi, const float* A_lo, long lon
   cudaStream_t s = (cudaStream_t)stream;
   if (a32) {
     switch (act_kind) {
-      case IMPFLOW_ACT_LIPSWISH: return launch_chain23<IMPFLOW_ACT_LIPSWISH, false, true>(maps, a, s);
-      case IMPFLOW_ACT_RELU: return launch_chain23<IMPFLOW_ACT_RELU, false, true>(maps, a, s);
-      case IMPFLOW_ACT_SIN: return launch_chain23<IMPFLOW_ACT_SIN, false, true>(maps, a, s);
-      default: return launch_chain23<IMPFLOW_ACT_NONE, false, true>(maps, a, s);
-    }
-  }
-  if (mc) {
-    switch (act_kind) {
-      case IMPFLOW_ACT_LIPSWISH: return launch_chain23<IMPFLOW_ACT_LIPSWISH, true, false>(maps, a, s);
-      case IMPFLOW_ACT_RELU: return launch_chain23<IMPFLOW_ACT_RELU, true, false>(maps, a, s);
-      case IMPFLOW_ACT_SIN: return launch_chain23<IMPFLOW_ACT_SIN, true, false>(maps, a, s);
-      default: return launch_chain23<IMPFLOW_ACT_NONE, true, false>(maps, a, s);
+      case IMPFLOW_ACT_LIPSWISH: return launch_chain23<IMPFLOW_ACT_LIPSWISH, true>(maps, a, s);
+      case IMPFLOW_ACT_RELU: return launch_chain23<IMPFLOW_ACT_RELU, true>(maps, a, s);
+      case IMPFLOW_ACT_SIN: return launch_chain23<IMPFLOW_ACT_SIN, true>(maps, a, s);
+      default: return launch_chain23<IMPFLOW_ACT_NONE, true>(maps, a, s);
     }
   }
   switch (act_kind) {
-    case IMPFLOW_ACT_LIPSWISH: return launch_chain23<IMPFLOW_ACT_LIPSWISH, false, false>(maps, a, s);
-    case IMPFLOW_ACT_RELU: return launch_chain23<IMPFLOW_ACT_RELU, false, false>(maps, a, s);
-    case IMPFLOW_ACT_SIN: return launch_chain23<IMPFLOW_ACT_SIN, false, false>(maps, a, s);
-    default: return launch_chain23<IMPFLOW_ACT_NONE, false, false>(maps, a, s);
+    case IMPFLOW_ACT_LIPSWISH: return launch_chain23<IMPFLOW_ACT_LIPSWISH, false>(maps, a, s);
+    case IMPFLOW_ACT_RELU: return launch_chain23<IMPFLOW_ACT_RELU, false>(maps, a, s);
+    case IMPFLOW_ACT_SIN: return launch_chain23<IMPFLOW_ACT_SIN, false>(maps, a, s);
+    default: return launch_chain23<IMPFLOW_ACT_NONE, false>(maps, a, s);
   }
 }

@@ -576,23 +576,16 @@ extern "C" int impflow_gemm_strided(const float* A, long long sAm, long long sAk
   return gemm_strided_simt(A, sAm, sAk, Bm, sBn, sBk, bias, out, ldc, M, N, K, (cudaStream_t)stream);
 }
 
-static int g_wide_tiles = 1;   // BN = 256 tiles for N >= 256 (halves the A-operand re-reads through L2)
 // Tile width: 256 halves the A-operand re-reads, but a problem with few row tiles fills more SMs (and
 // finishes in fewer, cheaper rounds) with 128-wide tiles: compare rounds x relative tile cost.
 static int tc_bn(int N, long long M = 1LL << 40) {
   if (N <= 32) return 32;
   if (N <= 64) return 64;
-  if (N < 256 || !g_wide_tiles) return 128;
+  if (N < 256) return 128;
   const long long m_tiles = (M + TC_BM - 1) / TC_BM;
   const long long r256 = (m_tiles * ((N + 255) / 256) + 147) / 148;
   const long long r128 = (m_tiles * ((N + 127) / 128) + 147) / 148;
   return (r128 * 55 < r256 * 100) ? 128 : 256;
-}
-
-extern "C" int impflow_gemm_tc_set_wide_tiles(int on) {
-  const int prev = g_wide_tiles;
-  g_wide_tiles = on ? 1 : 0;
-  return prev;
 }
 
 static int g_pair = 1;   // A/B switch (impflow_gemm_tc_set_pair)
@@ -600,7 +593,7 @@ static int g_pair = 1;   // A/B switch (impflow_gemm_tc_set_pair)
 // single CTAs: a pair tile streams 64 KB per CTA and K chunk (MMA-paced), a single 128 x 256 tile 96 KB
 // (about 1.5x the MMA time at the L2 -> SM rate), a 128 x 128 tile 64 KB for half the columns.
 static bool tc_use_pair(long long M, int N) {
-  if (!g_pair || !g_wide_tiles || N < 256) return false;
+  if (!g_pair || N < 256) return false;
   const long long n256 = (N + 255) / 256;
   const long long r_pair = (((M + 255) / 256) * n256 + 73) / 74;
   const long long m_tiles = (M + TC_BM - 1) / TC_BM;

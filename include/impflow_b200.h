@@ -91,15 +91,6 @@ int impflow_broyden_step(float* x_old, const float* g_old, const float* xn, cons
                          float* partial, impflow_broyden_state* state, int B, long long d, int threshold,
                          void* stream);
 
-/* A/B selection of the rank-1 update kernel (d % 4 == 0).  -1 or 0 (default) = two-pass cluster kernel (history read
- * for the dots, then again for the combinations; 16 independent loads per thread in flight); -3 = the same with 512
- * threads per CTA; -2 = history-streaming kernel: every history row crosses the SM boundary once ((6+2i) d 4 bytes per
- * sample, SURVEY 8(d)) — 1-D bulk copies into a shared-memory ring, per-row dots pushed into the peers' shared memory
- * of a <= 16-CTA cluster (d >= 2048); n > 0 = two passes in chunks of n rows whose second pass hits L2 (bit-identical
- * to the default).  Measured (B = 128, d = 65536): the default is the fastest; see csrc/broyden.cu.  Returns the
- * previous setting. */
-int impflow_broyden_set_chunk(int rows);
-
 /* Persistent small-d solver (toy / tabular MLP branches, d <= 128, widths <= 256): ONE cooperative
  * launch runs the whole solve of x_embed - f(z) - z = 0 — branch evaluations (fused fp32 MLP with the
  * activation `act_kind` between its L linear layers), batch-global norms, break rules, best iterate and
@@ -252,9 +243,6 @@ int impflow_gemm_nt_tc(const float* A_hi, const float* A_lo, long long lda, cons
  * epilogue (pre_out (+bias) only) and a workspace of impflow_gemm_tc_splits(M,N,K) * M * N floats the
  * kernel writes per-slice partials and a fixed-order reduce finishes; splitk_ws = NULL disables it. */
 int impflow_gemm_tc_splits(long long M, int N, int K);
-/* Tile-shape switch for A/B measurements: 1 (default) = 128x256 tiles when N >= 256, 0 = 128x128.
- * Returns the previous setting. */
-int impflow_gemm_tc_set_wide_tiles(int on);
 /* Epilogue switch for A/B measurements: 1 (default) = outputs staged in shared memory and written by bulk tensor
  * (TMA) stores, 0 = per-thread 32-byte global stores.  Returns the previous setting. */
 int impflow_gemm_tc_set_tma_store(int on);
@@ -312,10 +300,6 @@ int impflow_branch3_tc(const float* x0, long long ldx, const float* W1_hi, const
  * Needs C % 128 == 0 and 16-byte aligned rows (returns -2 otherwise).  Replaces two impflow_gemm_nt_tc launches and
  * the plane traffic between them. */
 int impflow_chain23_parts(int C);
-/* A/B switch: 1 (default) = with C = 512 the four quarter-CTAs of a row tile run as a thread-block cluster and share
- * the A1 chunks by TMA multicast; 0 (default: the lock-step of four SMs measured slower, 91 vs 123 TFLOP/s) =
- * independent CTAs.  Returns the previous setting. */
-int impflow_chain23_set_multicast(int on);
 /* A_lo = NULL: A_hi is the plain fp32 layer-2 input; the kernel splits every landed chunk into hi / lo on chip. */
 int impflow_chain23_tc(const float* A_hi, const float* A_lo, long long lda, const float* W2_hi, const float* W2_lo,
                        const float* W3_hi, const float* W3_lo, const float* bias2, const float* mul2, float* pre2_out,

@@ -1,5 +1,5 @@
 """Micro-benchmark of the fused layer-2+3 kernel (csrc/chain23_fused.cu) at the CIFAR scale-1 / scale-2 shapes, next
-to the two unfused tcgen05 GEMMs it replaces (CUDA events, L2 flushed).  `python scripts/chain23_bench.py [mc]`."""
+to the two unfused tcgen05 GEMMs it replaces (CUDA events, L2 flushed).  `python scripts/chain23_bench.py [a32]`."""
 import os
 import sys
 
@@ -10,8 +10,6 @@ import impflow_b200 as pkg  # noqa: E402
 
 ops = pkg.ops
 dev = torch.device('cuda')
-if 'mc' in sys.argv[1:]:
-    pkg._cabi.load().impflow_chain23_set_multicast(1)
 flush = torch.empty(64 * 1024 * 1024, device=dev)
 
 

@@ -1,7 +1,5 @@
-"""k_update (csrc/broyden.cu): the two-pass kernel (chunk 0), the history-streaming kernel (-2; -1 = automatic choice) and the
-L2-chunked kernel (n > 0).
-For each shape and chunk setting: n iterations of impflow_broyden_step on fixed random residuals, each timed alone
-(CUDA events, L2 flushed); the iterates and the history must be BIT-IDENTICAL across settings.
+"""k_update (csrc/broyden.cu): for each shape, n iterations of impflow_broyden_step on fixed random residuals, timed
+back to back (CUDA events between the iterations) and reported as a fraction of the HBM bandwidth.
 Usage: python scripts/update_bench.py [B d n_iter] ...   (default: the classifier and bench shapes)"""
 import ctypes
 import os
@@ -14,10 +12,9 @@ import impflow_b200 as pkg                                   # noqa: E402
 from impflow_b200.layers import broyden as _b                # noqa: E402
 
 
-def run(B, d, T, n_iter, chunk, flush, seed=0):
+def run(B, d, T, n_iter, seed=0):
     cabi = pkg._cabi
     lib = cabi.load()
-    lib.impflow_broyden_set_chunk(chunk)
     dev = torch.device('cuda')
     gen = torch.Generator(device='cuda').manual_seed(seed)
     wk = _b._workspace(B, d, T, dev)
@@ -30,34 +27,22 @@ def run(B, d, T, n_iter, chunk, flush, seed=0):
                                          vp(wk.low_sq), vp(wk.partial), vp(wk.state), B, d, T, 1e-30, cabi.stream()),
                'begin')
     x_old, xn = wk.xa, wk.xb
-    times = []
     evs = [torch.cuda.Event(enable_timing=True) for _ in range(n_iter + 1)]
-    if flush is None:
-        # back to back, as in the sync-free solver loop: the host runs ahead, the events sit between the iterations
-        # on the stream; nothing is flushed (a 2 GB history exceeds L2 by itself, the iterate / residual vectors were
-        # just written, as they are when a branch evaluation precedes the step)
-        torch.cuda.synchronize()
-        torch.cuda._sleep(2000000)            # keep the device busy while the host enqueues
-        evs[0].record()
+    # back to back, as in the sync-free solver loop: the host runs ahead, the events sit between the iterations on the
+    # stream; nothing is flushed (a 2 GB history exceeds L2 by itself, the iterate / residual vectors were just
+    # written, as they are when a branch evaluation precedes the step)
+    torch.cuda.synchronize()
+    torch.cuda._sleep(2000000)            # keep the device busy while the host enqueues
+    evs[0].record()
     for i in range(1, n_iter + 1):
         g_old, gn = gs[i - 1], gs[i]
-        if flush is not None:
-            flush.zero_()
-            evs[i - 1] = torch.cuda.Event(enable_timing=True)
-            evs[i - 1].record()
         cabi.check(lib.impflow_broyden_step(vp(x_old), vp(g_old), vp(xn), vp(gn), vp(wk.Ut), vp(wk.Vt), vp(wk.low_x),
                                             vp(wk.low_g), vp(wk.sample_sq), vp(wk.low_sq), vp(wk.partial),
                                             vp(wk.state), B, d, T, cabi.stream()), 'step')
         evs[i].record()
-        if flush is not None:
-            torch.cuda.synchronize()
-            times.append(evs[i - 1].elapsed_time(evs[i]) * 1e3)
         x_old, xn = xn, x_old
-    if flush is None:
-        torch.cuda.synchronize()
-        times = [evs[i - 1].elapsed_time(evs[i]) * 1e3 for i in range(1, n_iter + 1)]
-    lib.impflow_broyden_set_chunk(-1)
-    return times, (xn.clone(), wk.Ut[:, :n_iter].clone(), wk.Vt[:, :n_iter].clone())
+    torch.cuda.synchronize()
+    return [evs[i - 1].elapsed_time(evs[i]) * 1e3 for i in range(1, n_iter + 1)]
 
 
 def main():
@@ -65,27 +50,16 @@ def main():
     if len(sys.argv) > 3:
         a = [int(t) for t in sys.argv[1:]]
         shapes = [tuple(a[i:i + 3]) for i in range(0, len(a), 3)]
-    flush = torch.empty(64 * 1024 * 1024, device='cuda')
     hbm = 6543.1
     for B, d, n in shapes:
-        ref = None
-        for chunk, fl in ((0, None), (-3, None)):
-            run(B, d, 30, 2, chunk, fl)          # warm-up
-            times, out = run(B, d, 30, n, chunk, fl)
-            same = True if ref is None else all(torch.equal(a.view(torch.int32), b.view(torch.int32)) for a, b in zip(ref, out))
-            if not same:      # the streaming kernel slices the sample differently: agreement to round-off
-                same = 'max rel diff %.2e' % max(float((a - b).abs().max() / a.abs().max().clamp_min(1e-30))
-                                                 for a, b in zip(ref, out))
-            if ref is None:
-                ref = out
-            alg = [(6 + 2 * i) * d * 4.0 * B for i in range(1, n + 1)]
-            frac = [a / (t * 1e-6) / 1e9 / hbm for a, t in zip(alg, times)]
-            tot = sum(alg) / (sum(times) * 1e-6) / 1e9 / hbm
-            print('B=%d d=%d chunk=%2d %s bit-identical=%s  us/iter: %s  frac@i=1,4,8,%d: %.2f %.2f %.2f %.2f  overall %.3f'
-                  % (B, d, chunk, 'flushed' if fl is not None else 'back-to-back', same, ' '.join('%.0f' % t for t in times), n, frac[0], frac[3], frac[min(7, n - 1)],
-                     frac[-1], tot), flush=True)
-            del out
-        del ref
+        run(B, d, 30, 2)          # warm-up
+        times = run(B, d, 30, n)
+        alg = [(6 + 2 * i) * d * 4.0 * B for i in range(1, n + 1)]
+        frac = [a / (t * 1e-6) / 1e9 / hbm for a, t in zip(alg, times)]
+        tot = sum(alg) / (sum(times) * 1e-6) / 1e9 / hbm
+        print('B=%d d=%d back-to-back  us/iter: %s  frac@i=1,4,8,%d: %.2f %.2f %.2f %.2f  overall %.3f'
+              % (B, d, ' '.join('%.0f' % t for t in times), n, frac[0], frac[3], frac[min(7, n - 1)], frac[-1], tot),
+              flush=True)
         torch.cuda.empty_cache()
 
 

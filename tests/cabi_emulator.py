@@ -462,9 +462,6 @@ class EmulatedLib(object):
     def impflow_set_pdl(self, on):
         return 1
 
-    def impflow_gemm_tc_set_wide_tiles(self, on):
-        return 1
-
     def impflow_colsum(self, a, out, partial, M, N, stream):
         _f32(out, N)[:] = _f32(a, M * N).reshape(M, N).sum(0)
         self.launches += 1
@@ -640,12 +637,6 @@ class EmulatedLib(object):
 
     def impflow_conv3_set_chain23(self, on):
         return 1
-
-    def impflow_chain23_set_multicast(self, on):
-        return 1
-
-    def impflow_broyden_set_chunk(self, rows):
-        return -1
 
     def impflow_wgrad_set_slice_major(self, on):
         return 1
