@@ -39,6 +39,7 @@ import torch.nn as nn
 import torch.nn.functional as F
 
 from . import _cabi, ops
+from .layers import broyden as _broyden
 from .layers.base.activations import ReLU, Sin, Swish
 from .layers.base.mixed_lipschitz import InducedNormConv2d, InducedNormLinear, sigma_of
 
@@ -50,10 +51,12 @@ FUSED3 = {'on': True}
 # series / Broyden solve; off = the Python-driven launch sequences below.
 CONV3_NATIVE = {'on': True}
 
+# Every Broyden solve of a small MLP branch (forward / inverse and implicit backward) in one launch of the persistent
+# solver kernel (csrc/mlp_solver.cu); off = the generic kernel loop of layers/broyden.py.
+MLP_SOLVER = {'on': True}
+FUSED_SN_GRAD = {'on': True}     # weight-layout gradient + spectral chain in one C call
 # One-pass activation step of the Neumann reverse sweep (csrc/elementwise.cu: k_neumann_act_bwd); off = act_second +
 # two act_beta_grad + colsum + split.
-MLP_VJP_SOLVER = {'on': True}    # implicit backward of small MLP branches in the persistent solver kernel
-FUSED_SN_GRAD = {'on': True}     # weight-layout gradient + spectral chain in one C call
 NEUMANN_FUSED = {'on': True}
 
 # The same branch is evaluated at the same point several times per step (nnet_x(x) for x_embed, for the
@@ -269,43 +272,48 @@ class BranchProgram(object):
         self._key, self._weights = key, ws
         return ws
 
-    def mlp_solver_spec(self, x):
-        """Arguments of the persistent small-d solver (csrc/mlp_solver.cu) or None if this branch does not
-        qualify: plain Linear/act/.../Linear MLP, one activation kind, d <= 128, widths <= 256."""
-        if not self.is_linear or self.post_act is not None or self.stages[0][0] is not None:
+    def _mlp_weights(self, M):
+        """(effective weights, widths [d, h_1, ..., d]) of a branch the persistent small-d kernels (csrc/mlp_solver.cu)
+        take at M rows: Linear act Linear ... act Linear with no leading or trailing activation, d <= 128, widths <=
+        256, at most 8 layers.  None for any other branch."""
+        if not self.is_linear or self.post_act is not None or self.stages[0][0] is not None \
+                or any(a is None for a, _ in self.stages[1:]):
             return None
-        if any(a is None for a, _ in self.stages[1:]):
-            return None
-        kinds = {a.kind for a, _ in self.stages[1:]}
-        if len(kinds) > 1:
-            return None
-        rows, meta = self._to_rows(x)
-        ws = self._prep(rows.shape[0], meta)
+        ws = self._prep(M)
         dims = [ws[0].cin] + [w.cout for w in ws]
         if dims[0] != dims[-1] or dims[0] > 128 or max(dims) > 256 or len(ws) > 8:
             return None
-        key = ('mlp', self._key)
+        return ws, dims
+
+    def _mlp_wt(self):
+        """The effective weights transposed to (in, out), as the kernels' forward evaluation reads them; cached until
+        the weights change."""
         cached = getattr(self, '_mlp_spec', None)
-        if cached is None or cached[0] != key:
-            Wt = [w.fwd[:, :w.cin].t().contiguous() for w in ws]
-            cached = self._mlp_spec = (key, Wt)
+        if cached is None or cached[0] != self._key:
+            cached = self._mlp_spec = (self._key, [w.fwd[:, :w.cin].t().contiguous() for w in self._weights])
+        return cached[1]
+
+    def mlp_solver_spec(self, x):
+        """Arguments of the persistent solver's forward / inverse mode (impflow_mlp_broyden_solve) for inputs shaped
+        like x, or None if the branch does not qualify (_mlp_weights, and one activation kind throughout)."""
+        if not MLP_SOLVER['on'] or not self.is_linear or len({a.kind for a, _ in self.stages[1:] if a is not None}) > 1:
+            return None
+        fit = self._mlp_weights(self._to_rows(x)[0].shape[0])
+        if fit is None:
+            return None
+        ws, dims = fit
         acts = [a for a, _ in self.stages[1:]]          # acts[l] sits behind layer l; each Swish owns its beta
         kind = acts[0].kind if acts else ops.ACT_NONE
         betas = [a.beta_sp() for a in acts] if kind == ops.ACT_LIPSWISH else None
-        return (cached[1], [w.bias for w in ws], dims, kind, betas)
+        return (self._mlp_wt(), [w.bias for w in ws], dims, kind, betas)
 
-    def mlp_vjp_spec(self, saved):
-        """Arguments of the persistent solver's implicit-backward mode (impflow_mlp_broyden_solve_vjp) at the point
-        of `saved`, or None if the branch does not qualify (same conditions as mlp_solver_spec)."""
-        if not MLP_VJP_SOLVER['on'] or not self.is_linear or self.post_act is not None \
-                or self.stages[0][0] is not None:
+    def _mlp_vjp_operands(self, saved):
+        """(effective weights [out][ld], their row strides, act' multipliers (None for layer 0), dims) of the
+        persistent kernels' vjp mode at the point of `saved`, or None if the branch does not qualify."""
+        fit = self._mlp_weights(saved.M)
+        if fit is None:
             return None
-        if any(a is None for a, _ in self.stages[1:]):
-            return None
-        ws = self._prep(saved.M)
-        dims = [ws[0].cin] + [w.cout for w in ws]
-        if dims[0] != dims[-1] or dims[0] > 128 or max(dims) > 256 or len(ws) > 8:
-            return None
+        ws, dims = fit
         if any(w.fwd is None or w.fwd.stride(1) != 1 for w in ws):
             return None
         dmul = [None] + [self._deriv(saved, i).contiguous() for i in range(1, len(ws))]
@@ -313,19 +321,21 @@ class BranchProgram(object):
             return None
         return [w.fwd for w in ws], [w.fwd.stride(0) for w in ws], dmul, dims
 
+    def mlp_vjp_spec(self, saved):
+        """Arguments of the persistent solver's implicit-backward mode (impflow_mlp_broyden_solve_vjp) at the point
+        of `saved`, or None if the branch does not qualify."""
+        return self._mlp_vjp_operands(saved) if MLP_SOLVER['on'] else None
+
     def mlp_series_spec(self, saved):
         """Arguments of the one-launch MLP power series (impflow_mlp_series) at the point of `saved`, or None if the
-        branch does not qualify (same conditions as the persistent solver)."""
-        vs = self.mlp_vjp_spec(saved) if MLP_SERIES['on'] else None
+        branch does not qualify: the kernel takes (samples, d) inputs.  Its 1..32 terms are the caller's to check."""
+        if not MLP_SERIES['on'] or saved.meta[0] != 'lin' or len(saved.meta[1]) != 2:
+            return None
+        vs = self._mlp_vjp_operands(saved)
         if vs is None:
             return None
         W, ldw, dmul, dims = vs
-        ws = self._prep(saved.M)
-        key = ('mlp', self._key)
-        cached = getattr(self, '_mlp_spec', None)
-        if cached is None or cached[0] != key:
-            cached = self._mlp_spec = (key, [w.fwd[:, :w.cin].t().contiguous() for w in ws])
-        return W, ldw, cached[1], dmul, dims
+        return W, ldw, self._mlp_wt(), dmul, dims
 
     # ---------------------------------------------------------------- plumbing
     def _to_rows(self, x):
@@ -567,11 +577,15 @@ class BranchProgram(object):
         return self._conv3(self._prep(x.shape[0] * x.shape[2] * x.shape[3], meta), meta)
 
     def neumann_chain(self, saved, vareps, coeffs):
-        """w = v + sum_k coeffs[k-1] v^T J^k in one C call (implicit_block.py:431-435), or None if this
-        branch has no native plan."""
+        """w = v + sum_k coeffs[k-1] v^T J^k (implicit_block.py:431-435): one C call with a native plan, else a chain
+        of vjp evaluations."""
         P = self._conv3(self._prep(saved.M), saved.meta)
         if P is None:
-            return None
+            vjp = w = vareps
+            for c in coeffs:
+                vjp = self.vjp(vjp, saved)
+                w = ops.lincomb3(w, 1.0, vjp, c)
+            return w
         t, _ = self._to_rows(vareps)
         w_rows = torch.empty_like(t)
         n = len(coeffs)
@@ -586,10 +600,16 @@ class BranchProgram(object):
 
     def hutchinson_series(self, saved, vareps, dot_coeffs):
         """sum_k dot_coeffs[k-1] <v^T J^k, v> per sample — the basic estimator's no-graph form (eval mode,
-        implicit_block.py:418-426) — in one C call, or None if this branch has no native plan."""
+        implicit_block.py:418-426): one C call with a native plan, else a chain of vjp evaluations and row dots
+        accumulated in place."""
         P = self._conv3(self._prep(saved.M), saved.meta)
         if P is None:
-            return None
+            out = torch.zeros(vareps.shape[0], device=vareps.device, dtype=torch.float32)
+            vjp = vareps
+            for c in dot_coeffs:
+                vjp = self.vjp(vjp, saved)
+                ops.rowdot(vjp, vareps, out=out, alpha=float(c), beta=1.0)
+            return out
         t, _ = self._to_rows(vareps)
         n = len(dot_coeffs)
         out = torch.empty(vareps.shape[0], device=t.device, dtype=torch.float32)
@@ -602,42 +622,55 @@ class BranchProgram(object):
             self._record_conv3(P, True, False, n)
         return out
 
-    def broyden_solve(self, mode, rhs, saved, threshold, eps):
-        """Whole Broyden solve in one C call (mode 0: rhs - nnet(z) - z = 0 from z = 0; mode 1:
-        v^T J + v - rhs = 0 at `saved`).  Returns the reference's result dict, or None without a plan."""
-        from .layers import broyden as _b
-        B = rhs.shape[0]
-        meta = ('conv', (B, rhs.shape[2], rhs.shape[3])) if rhs.dim() == 4 else None
-        if meta is None:
-            return None
-        M = B * rhs.shape[2] * rhs.shape[3]
-        P = self._conv3(self._prep(M, meta), meta)
-        if P is None:
-            return None
-        lib = _cabi.load()
-        rows, _ = self._to_rows(rhs)
-        d = rows.numel() // B
-        eps_scaled = eps * (B * d) ** 0.5
-        wk = _b._workspace(B, d, threshold, rows.device)
-        if not hasattr(wk, 'ga'):
-            wk.ga = torch.empty(B, d, device=rows.device, dtype=torch.float32)
-            wk.gb = torch.empty(B, d, device=rows.device, dtype=torch.float32)
-        wk.xa.zero_()
-        if mode == 1:
-            pre0, d1, d2 = self._vjp_operands(saved, P)
+    def solve(self, mode, rhs, saved, threshold, eps):
+        """Broyden solve of this branch's implicit equation, with rhs and result in module layout.
+        Mode 0: rhs - nnet(z) - z = 0 from z = 0 (forward / inverse, implicit_block.py:68-80); mode 1: v^T J + v - rhs
+        = 0 at the point of `saved` from v = 0 (implicit backward, :199-207).  Returns the reference's result dict
+        (broyden.py:184-193).
+
+        The whole solve is one call where the branch allows it: the persistent kernel of a small MLP branch
+        (csrc/mlp_solver.cu), or the native runtime of a 3-layer conv branch (csrc/conv3_plan.cu).  Otherwise the
+        generic kernel loop of layers/broyden.py iterates in rows layout, which for a conv branch saves the NCHW <->
+        NHWC copies of every evaluation: a sample is a contiguous block either way, and the solver's per-sample dots
+        and norms do not depend on the order inside it.  For an MLP branch rows layout is module layout."""
+        if mode == 0:
+            spec = self.mlp_solver_spec(rhs)
+            if spec is not None:
+                return _broyden.broyden_mlp(spec, rhs, torch.zeros_like(rhs), threshold, eps)
         else:
-            pre0 = d1 = d2 = None
-        vp = lambda t: ctypes.c_void_p(t.data_ptr())
-        _cabi.check(lib.impflow_conv3_broyden(
-            self._plan_ptr(P), mode, _cabi.ptr(rows), pre0, d1, d2, vp(wk.xa), vp(wk.xb), vp(wk.ga), vp(wk.gb),
-            vp(wk.low_x), vp(wk.low_g), vp(wk.Ut), vp(wk.Vt), vp(wk.sample_sq), vp(wk.low_sq), vp(wk.partial),
-            vp(wk.state), vp(wk.state_host), threshold, float(eps_scaled), _cabi.stream()), 'conv3_broyden')
-        best = wk.low_x.clone()         # first: the stream is empty after the solve, host work comes after the launch
-        state = wk.host_state()
-        info = _b._result_dict(wk, state, (B, d), eps_scaled, threshold, result=best)
-        info['result'] = self._from_rows(info['result'].view(M, P.c), meta)
-        if ops.GEMM_PROFILE['on']:
-            self._record_conv3(P, mode == 1, False, info['nstep'] + 1)
+            spec = self.mlp_vjp_spec(saved)
+            if spec is not None:
+                return _broyden.broyden_mlp_vjp(spec, rhs, threshold, eps)
+        P = self.native_plan(rhs)
+        rows, meta = self._to_rows(rhs)
+        B, M = rhs.shape[0], rows.shape[0]
+        d = rows.numel() // B
+        if P is not None:
+            eps_scaled = _broyden.scaled_eps(eps, B, d)
+            wk = _broyden._workspace(B, d, threshold, rows.device)
+            wk.one_call_buffers()
+            wk.xa.zero_()
+            pre0, d1, d2 = self._vjp_operands(saved, P) if mode == 1 else (None, None, None)
+            vp = lambda t: ctypes.c_void_p(t.data_ptr())
+            _cabi.check(_cabi.load().impflow_conv3_broyden(
+                self._plan_ptr(P), mode, _cabi.ptr(rows), pre0, d1, d2, vp(wk.xa), vp(wk.xb), vp(wk.ga), vp(wk.gb),
+                vp(wk.low_x), vp(wk.low_g), vp(wk.Ut), vp(wk.Vt), vp(wk.sample_sq), vp(wk.low_sq), vp(wk.partial),
+                vp(wk.state), vp(wk.state_host), threshold, float(eps_scaled), _cabi.stream()), 'conv3_broyden')
+            best = wk.low_x.clone()     # first: the stream is empty after the solve, host work comes after the launch
+            info = _broyden._result_dict(wk, wk.host_state(), (B, d), eps_scaled, threshold, result=best)
+            if ops.GEMM_PROFILE['on']:
+                self._record_conv3(P, mode == 1, False, info['nstep'] + 1)
+        else:
+            if mode == 0:
+                def g(z2d):
+                    zr = z2d.view(M, -1)
+                    return ops.lincomb3(rows, 1.0, self.forward_rows(zr, meta), -1.0, zr, -1.0).view(B, -1)
+            else:
+                def g(v2d):
+                    vr = v2d.view(M, -1)
+                    return ops.lincomb3(self.vjp_rows(vr, saved), 1.0, vr, 1.0, rows, -1.0).view(B, -1)
+            info = _broyden.broyden(g, torch.zeros(B, d, device=rows.device), threshold, eps)
+        info['result'] = self._from_rows(info['result'].view(M, -1), meta)
         return info
 
     def _ains(self, saved):

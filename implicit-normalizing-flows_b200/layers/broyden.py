@@ -5,6 +5,7 @@ solver algebra (rank-1 updates, low-rank mat-vecs, norms, best-iterate tracking,
 runs in the impflow CUDA kernels with the bookkeeping kept on the device.  The host reads a
 600-byte state record per iteration to learn whether the loop continues."""
 import ctypes
+import math
 
 import numpy as np
 import torch
@@ -43,6 +44,16 @@ class _Workspace(object):
         # progress records the sync-free conv solver polls (impflow_conv3_broyden_host_bytes)
         self.state_nbytes = nbytes
         self.state_host = _cabi.pinned_bytes(max(nbytes, int(lib.impflow_conv3_broyden_host_bytes(T))))
+        self.ga = self.gb = self.partial_d = None
+
+    def one_call_buffers(self, mlp=False):
+        """Allocate on first use what the one-call solvers need beyond the generic loop's buffers: the residual pair
+        ga / gb and, for the persistent MLP kernel (mlp=True), its fp64 partial sums."""
+        if self.ga is None:
+            self.ga, self.gb = torch.empty_like(self.xa), torch.empty_like(self.xa)
+        if mlp and self.partial_d is None:
+            self.partial_d = torch.empty(int(_cabi.load().impflow_mlp_solver_partial_doubles()), device=self.xa.device,
+                                         dtype=torch.float64)
 
     def read_state(self):
         self.state_host[:self.state_nbytes].copy_(self.state, non_blocking=True)
@@ -61,6 +72,11 @@ def _workspace(B, d, T, device):
             _workspaces.clear()
         ws = _workspaces[key] = _Workspace(B, d, T, device)
     return ws
+
+
+def scaled_eps(eps, B, d):
+    """The stopping tolerance of a solve on the norm of the whole (B, d) residual (broyden.py:131)."""
+    return eps * math.sqrt(B * d)
 
 
 def _result_dict(ws, state, shape, eps_scaled, threshold, result=None):
@@ -90,13 +106,9 @@ def broyden_mlp(spec, x_embed, z0, threshold, eps):
     B = shape[0]
     d = z0.numel() // B
     assert d == dims[0] == dims[-1]
-    eps_scaled = eps * np.sqrt(np.prod((B, d)))
+    eps_scaled = scaled_eps(eps, B, d)
     ws = _workspace(B, d, threshold, z0.device)
-    if not hasattr(ws, 'gb'):
-        ws.ga = torch.empty(B, d, device=z0.device, dtype=torch.float32)
-        ws.gb = torch.empty(B, d, device=z0.device, dtype=torch.float32)
-        ws.partial_d = torch.empty(int(lib.impflow_mlp_solver_partial_doubles()), device=z0.device,
-                                   dtype=torch.float64)
+    ws.one_call_buffers(mlp=True)
     ws.xa.copy_(z0.reshape(B, d))
     L = len(Wt)
     wt_arr = (ctypes.c_void_p * L)(*[w.data_ptr() for w in Wt])
@@ -129,13 +141,9 @@ def broyden_mlp_vjp(spec, rhs, threshold, eps):
     B = shape[0]
     d = rhs.numel() // B
     assert d == dims[0] == dims[-1]
-    eps_scaled = eps * np.sqrt(np.prod((B, d)))
+    eps_scaled = scaled_eps(eps, B, d)
     ws = _workspace(B, d, threshold, rhs.device)
-    if not hasattr(ws, 'gb'):
-        ws.ga = torch.empty(B, d, device=rhs.device, dtype=torch.float32)
-        ws.gb = torch.empty(B, d, device=rhs.device, dtype=torch.float32)
-        ws.partial_d = torch.empty(int(lib.impflow_mlp_solver_partial_doubles()), device=rhs.device,
-                                   dtype=torch.float64)
+    ws.one_call_buffers(mlp=True)
     ws.xa.zero_()
     L = len(W)
     w_arr = (ctypes.c_void_p * L)(*[w.data_ptr() for w in W])
@@ -163,7 +171,7 @@ def broyden(g_, x0, threshold, eps, ls=False, name='unknown'):
     shape = x0.shape
     B = shape[0]
     d = x0.numel() // B
-    eps_scaled = eps * np.sqrt(np.prod((B, d)))       # broyden.py:131
+    eps_scaled = scaled_eps(eps, B, d)
     ws = _workspace(B, d, threshold, x0.device)
     st = _cabi.stream
 

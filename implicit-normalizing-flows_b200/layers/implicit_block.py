@@ -21,7 +21,7 @@ from torch.autograd import Function
 
 from .. import ops
 from ..parallel import sink_grads
-from .broyden import broyden, broyden_mlp, broyden_mlp_vjp
+from .broyden import broyden
 
 __all__ = ['imBlock']
 
@@ -34,8 +34,6 @@ PROBE_MODE = {'mode': 'reference'}
 # the vjps of the implicit backward solve and of the Neumann / eval-mode power series.  Off = every
 # branch evaluation goes through the module and autograd (same kernels, many more launches).
 FUSED = {'on': True}
-# One-launch persistent solver for small-d MLP branches (csrc/mlp_solver.cu); off = host-driven loop.
-PERSISTENT_MLP = {'on': True}
 
 
 def _program(nnet):
@@ -108,7 +106,6 @@ def _timed(kind, like, fn):
 
 # Independent halves of a block's work (the log-det estimates of the x- and z-branch) on two streams.
 OVERLAP = {'on': True}
-ROWS_SOLVE = {'on': True}      # generic Broyden loop of a conv branch iterates in rows (NHWC) layout
 HOST_AHEAD = {'on': True}     # imBlock.forward: twin refresh and random draws in front of the forward solve
 _side = {}
 
@@ -256,28 +253,9 @@ class RootFind(Function):
         eps, threshold = args[-2], args[-1]
         x_embed = ops.lincomb3(branch_eval(nnet_x, x, keep=getattr(nnet_x, 'training', False)), 1.0, x, 1.0)
         prog_z = _program(nnet_z)
-        spec = prog_z.mlp_solver_spec(z0) if (prog_z is not None and PERSISTENT_MLP['on']) else None
-        info = None
-        if spec is not None:
-            # small-d MLP branch: the whole solve (branch evaluations included) in one persistent kernel
-            info = broyden_mlp(spec, x_embed, torch.zeros_like(z0), threshold, eps)
-        elif prog_z is not None:
-            # conv branch: the whole solve in one call of the native runtime (csrc/conv3_plan.cu)
-            info = prog_z.broyden_solve(0, x_embed, None, threshold, eps)
-        if info is None and prog_z is not None and not prog_z.is_linear and x_embed.dim() == 4 and ROWS_SOLVE['on']:
-            # conv branch without a native plan (classifier: 3x3 - 3x3): iterate in rows (NHWC) layout, no layout copy
-            # per evaluation (the solver's per-sample dots and norms do not depend on the order inside a sample)
-            rows_e, meta = prog_z._to_rows(x_embed)
-            B, M = x_embed.shape[0], rows_e.shape[0]
-
-            def g_rows(z2d):
-                zr = z2d.view(M, -1)
-                return ops.lincomb3(rows_e, 1.0, prog_z.forward_rows(zr, meta), -1.0, zr, -1.0).view(B, -1)
-
-            info = broyden(g_rows, torch.zeros(B, rows_e.numel() // B, device=x_embed.device), threshold=threshold,
-                           eps=eps, name='forward')
-            info['result'] = prog_z._from_rows(info['result'].view(M, -1), meta)
-        if info is None:
+        if prog_z is not None:
+            info = prog_z.solve(0, x_embed, None, threshold, eps)
+        else:
             def g(z):     # x_embed - nnet_z(z) - z in one kernel (implicit_block.py:72)
                 return ops.lincomb3(x_embed, 1.0, branch_eval(nnet_z, z), -1.0, z, -1.0)
 
@@ -376,28 +354,7 @@ class imBlock(nn.Module):
                     _, saved_x = prog_x.forward_saved(xa)
                     prog_x.prepare_vjp(saved_x)
 
-                    def solve():
-                        info = prog_z.broyden_solve(1, grad, saved_z, threshold, eps)
-                        if info is None:
-                            spec = prog_z.mlp_vjp_spec(saved_z)
-                            if spec is not None:       # small-d MLP: the whole solve in one persistent kernel
-                                info = broyden_mlp_vjp(spec, grad, threshold, eps)
-                        if info is None and not prog_z.is_linear and grad.dim() == 4 and ROWS_SOLVE['on']:
-                            grows, meta = prog_z._to_rows(grad)          # rows-layout iteration, see RootFind
-                            B, M = grad.shape[0], grows.shape[0]
-
-                            def g_rows(v2d):
-                                vr = v2d.view(M, -1)
-                                return ops.lincomb3(prog_z.vjp_rows(vr, saved_z), 1.0, vr, 1.0, grows, -1.0).view(B, -1)
-
-                            info = broyden(g_rows, torch.zeros(B, grows.numel() // B, device=grad.device),
-                                           threshold=threshold, eps=eps, name='backward')
-                            info['result'] = prog_z._from_rows(info['result'].view(M, -1), meta)
-                        if info is None:
-                            info = broyden(lambda v: ops.lincomb3(prog_z.vjp(v, saved_z), 1.0, v, 1.0, grad, -1.0),
-                                           torch.zeros_like(grad), threshold=threshold, eps=eps, name='backward')
-                        return info
-                    info = _timed('bwd', grad, solve)
+                    info = _timed('bwd', grad, lambda: prog_z.solve(1, grad, saved_z, threshold, eps))
                     imBlock.Backward.last_info = info
                     if ctx.stats is not None:
                         ctx.stats['bwd'] = info
@@ -654,13 +611,7 @@ class MemoryEfficientLogDetEstimator(torch.autograd.Function):
             xd = x.detach()
             _, saved = prog.forward_saved(xd)
             coeffs = [float((-1) ** k * coeff_fn(k)) for k in range(1, n_power_series + 1)]
-            neumann_vjp = prog.neumann_chain(saved, vareps, coeffs)       # one C call when native
-            if neumann_vjp is None:
-                vjp = neumann_vjp = vareps
-                for k in range(1, n_power_series + 1):
-                    vjp = prog.vjp(vjp, saved)
-                    neumann_vjp = ops.lincomb3(neumann_vjp, 1.0, vjp, coeffs[k - 1])
-            return prog.neumann(saved, neumann_vjp, vareps)
+            return prog.neumann(saved, prog.neumann_chain(saved, vareps, coeffs), vareps)
 
     @staticmethod
     def forward(ctx, estimator_fn, gnet, x, n_power_series, vareps, coeff_fn, training, payload, *g_params):
@@ -766,7 +717,7 @@ class _GraphFreeBasic(Function):
         xd = x.detach()
         _, saved = prog.forward_saved(xd)
         ctx.series = None
-        spec = prog.mlp_series_spec(saved) if (xd.dim() == 2 and 1 <= len(coeffs) <= 32) else None
+        spec = prog.mlp_series_spec(saved) if 1 <= len(coeffs) <= 32 else None
         if spec is not None:
             # small-d MLP branch: both chains, the combinations and the estimate in ONE launch (k_mlp_series)
             out, _, Rs, Wm = ops.mlp_series(spec, vareps, coeffs)
@@ -837,25 +788,16 @@ class _GraphFreeBasic(Function):
 
 def basic_logdet_estimator(g, x, n_power_series, vareps, coeff_fn, training, program=None):
     """sum_k (-1)^(k+1)/k coeff(k) <v^T J^k, v>  (implicit_block.py:418-426)."""
-    vjp = vareps
     if not training and program is not None:
-        # eval mode builds no graph: the whole chain runs on the fused vjp kernels, the Hutchinson
-        # dots accumulate in place
+        # eval mode builds no graph: the whole chain runs on the fused vjp kernels
         with torch.no_grad():
             _, saved = program.forward_saved(x.detach())
-            program._saved = saved
-            dots = program.hutchinson_series(saved, vareps, [(-1) ** (k + 1) / k * coeff_fn(k)
-                                                              for k in range(1, n_power_series + 1)])
-            if dots is not None:        # conv branch: the whole chain and its dots in one C call
-                return dots
-            out = torch.zeros(x.shape[0], device=x.device, dtype=torch.float32)
-            for k in range(1, n_power_series + 1):
-                vjp = program.vjp(vjp)
-                ops.rowdot(vjp, vareps, out=out, alpha=float((-1) ** (k + 1) / k * coeff_fn(k)), beta=1.0)
-        return out
+            return program.hutchinson_series(saved, vareps, [(-1) ** (k + 1) / k * coeff_fn(k)
+                                                             for k in range(1, n_power_series + 1)])
     if training and program is not None and GRAPH_FREE_BASIC['on'] and n_power_series >= 1:
         coeffs = [(-1) ** (k + 1) / k * coeff_fn(k) for k in range(1, n_power_series + 1)]
         return _GraphFreeBasic.apply(x, program, vareps, coeffs, *program.params)
+    vjp = vareps
     logdetgrad = torch.zeros((), device=x.device, dtype=x.dtype)
     for k in range(1, n_power_series + 1):
         with ops.activations_only():

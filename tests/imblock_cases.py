@@ -578,7 +578,7 @@ def case_mlp_solver_per_layer_beta():
     inverse solves of an MLP imBlock with diverged betas, persistent kernel vs the host-driven loop."""
     pkg = _pkg()
     layers = pkg.layers
-    from impflow_b200.layers import implicit_block
+    from impflow_b200 import branch_program
     dev = DEV['device']
     torch.manual_seed(21)
     d, dims = 6, [6, 32, 32, 32, 6]
@@ -605,14 +605,14 @@ def case_mlp_solver_per_layer_beta():
     x = torch.randn(64, d, device=dev)
     outs = {}
     for persistent in (True, False):
-        implicit_block.PERSISTENT_MLP['on'] = persistent
+        branch_program.MLP_SOLVER['on'] = persistent
         try:
             with torch.no_grad():
                 z = blk(x)
                 xr = blk.inverse(z)
             outs[persistent] = (z.cpu(), xr.cpu(), blk.solver_stats['fwd']['nstep'], blk.solver_stats['inv']['nstep'])
         finally:
-            implicit_block.PERSISTENT_MLP['on'] = True
+            branch_program.MLP_SOLVER['on'] = True
     a, b = outs[True], outs[False]
     assert a[2] == b[2] and a[3] == b[3], (a[2:], b[2:])
     assert rel_err(a[0], b[0]) < 1e-5 and rel_err(a[1], b[1]) < 1e-5

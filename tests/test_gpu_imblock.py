@@ -182,20 +182,20 @@ def test_mlp_backward_solve_runs_in_the_persistent_kernel(golden, monkeypatch):
     """The implicit backward of a small MLP imBlock is ONE solver launch (impflow_mlp_broyden_solve_vjp), with the
     golden iteration counts and gradients; switched off, the host-driven loop gives the same answer."""
     from impflow_b200 import branch_program
-    from impflow_b200.layers import implicit_block
+    from impflow_b200.layers import broyden
     calls = []
-    orig = implicit_block.broyden_mlp_vjp
+    orig = broyden.broyden_mlp_vjp
 
     def counted(*a, **k):
         calls.append(1)
         return orig(*a, **k)
-    monkeypatch.setattr(implicit_block, 'broyden_mlp_vjp', counted)
+    monkeypatch.setattr(broyden, 'broyden_mlp_vjp', counted)
     cases.case_imblock_mlp_train(golden, 'tab6')
     assert len(calls) >= 1
     n = len(calls)
-    branch_program.MLP_VJP_SOLVER['on'] = False
+    branch_program.MLP_SOLVER['on'] = False
     try:
         cases.case_imblock_mlp_train(golden, 'tab6')
     finally:
-        branch_program.MLP_VJP_SOLVER['on'] = True
+        branch_program.MLP_SOLVER['on'] = True
     assert len(calls) == n

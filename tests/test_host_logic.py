@@ -211,7 +211,7 @@ def test_fused3_tile_kernel_is_taken():
     assert branch_cases.case_fused3_is_taken('cifar_lead') == 0        # width 32: three GEMMs
 
 
-def test_fused_paths_are_taken(golden, monkeypatch):
+def test_fused_paths_are_taken(golden, monkeypatch, _emulated):
     """Guards against silently falling back to the module/autograd path: one CIFAR-style training
     forward+backward must run the Neumann gradient, the attach backward and all vjps on the
     graph-free branch programs and never build an autograd graph through the branch."""
@@ -224,15 +224,15 @@ def test_fused_paths_are_taken(golden, monkeypatch):
     def wrap(cls, name, key):
         orig = getattr(cls, name)
 
-        def f(self, *a, **k):
+        def f(*a, **k):
             counts[key] += 1
-            return orig(self, *a, **k)
+            return orig(*a, **k)
         monkeypatch.setattr(cls, name, f)
     wrap(bp.BranchProgram, 'neumann', 'neumann')
     wrap(bp.BranchProgram, 'backward_full', 'backward_full')
     wrap(bp.BranchProgram, 'vjp', 'vjp')
-    wrap(bp.BranchProgram, 'neumann_chain', 'chain')
-    wrap(bp.BranchProgram, 'broyden_solve', 'solve')
+    wrap(_emulated, 'impflow_conv3_power_series', 'chain')
+    wrap(_emulated, 'impflow_conv3_broyden', 'solve')
     orig_est = ib.neumann_logdet_estimator
     monkeypatch.setattr(ib, 'neumann_logdet_estimator',
                         lambda *a, **k: (counts.__setitem__('autograd_estimator', counts['autograd_estimator'] + 1),
@@ -337,21 +337,21 @@ def test_mlp_backward_solve_runs_in_the_persistent_kernel(golden, monkeypatch):
     """The implicit backward of a small MLP imBlock is ONE solver launch (impflow_mlp_broyden_solve_vjp), with the
     golden iteration counts and gradients; switched off, the host-driven loop gives the same answer."""
     from impflow_b200 import branch_program
-    from impflow_b200.layers import implicit_block
+    from impflow_b200.layers import broyden
     from tests import imblock_cases
     calls = []
-    orig = implicit_block.broyden_mlp_vjp
+    orig = broyden.broyden_mlp_vjp
 
     def counted(*a, **k):
         calls.append(1)
         return orig(*a, **k)
-    monkeypatch.setattr(implicit_block, 'broyden_mlp_vjp', counted)
+    monkeypatch.setattr(broyden, 'broyden_mlp_vjp', counted)
     imblock_cases.case_imblock_mlp_train(golden, 'tab6')
     assert len(calls) >= 1
     n = len(calls)
-    branch_program.MLP_VJP_SOLVER['on'] = False
+    branch_program.MLP_SOLVER['on'] = False
     try:
         imblock_cases.case_imblock_mlp_train(golden, 'tab6')
     finally:
-        branch_program.MLP_VJP_SOLVER['on'] = True
+        branch_program.MLP_SOLVER['on'] = True
     assert len(calls) == n
