@@ -333,6 +333,42 @@ def test_actnorm_fused_matches_expression():
     imblock_cases.case_actnorm_fused_matches_expression()
 
 
+@pytest.mark.parametrize('mode', [0, 1])
+@pytest.mark.parametrize('name', ['tile', 'chain23_8', 'gemm3_3'])
+def test_solve_conv_vs_oracle(name, mode):
+    """The solver-level cases of test_gpu_solve.py at small shapes: one-call conv solve against the float64 oracle."""
+    from tests import solve_cases
+    solve_cases.case_conv_vs_oracle(name, mode)
+
+
+@pytest.mark.parametrize('mode', [0, 1])
+@pytest.mark.parametrize('rule', ['cap', 'cap_roundoff', 'prot_break', 'zero_rows'])
+def test_solve_conv_stopping_rules(rule, mode):
+    from tests import solve_cases
+    solve_cases.case_conv_stop(rule, 'tile_small', mode)
+
+
+@pytest.mark.parametrize('mode', [0, 1])
+@pytest.mark.parametrize('rule', ['cap', 'cap_roundoff', 'prot_break'])
+def test_solve_mlp_stopping_rules(rule, mode):
+    from tests import solve_cases
+    solve_cases.case_mlp_stop(rule, mode)
+
+
+def test_solve_mlp_vjp_and_limits():
+    from tests import solve_cases
+    solve_cases.case_mlp_stop('zero_rows', 1)
+    solve_cases.case_mlp_vjp('b1')
+    solve_cases.case_mlp_vjp('relu43')
+    solve_cases.case_mlp_beyond_limits('d129')
+
+
+@pytest.mark.parametrize('solver', ['conv', 'mlp', 'rows'])
+def test_solve_back_to_back_on_one_workspace(solver):
+    from tests import solve_cases
+    solve_cases.case_back_to_back(solver)
+
+
 def test_mlp_backward_solve_runs_in_the_persistent_kernel(golden, monkeypatch):
     """The implicit backward of a small MLP imBlock is ONE solver launch (impflow_mlp_broyden_solve_vjp), with the
     golden iteration counts and gradients; switched off, the host-driven loop gives the same answer."""
