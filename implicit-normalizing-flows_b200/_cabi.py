@@ -30,6 +30,7 @@ SIGNATURES = {
     'impflow_mlp_solver_partial_doubles': (ctypes.c_size_t, []),
     'impflow_mlp_broyden_solve': (_i, [_c_fp, _c_fp, _c_fp, _c_fp, _i, _i, _c_fp] + [_c_fp] * 12 + [_i, _i, _d, _c_fp]),
     'impflow_mlp_broyden_solve_vjp': (_i, [_c_fp, _c_fp, _c_fp, _c_fp, _c_fp, _i] + [_c_fp] * 12 + [_i, _i, _d, _c_fp]),
+    'impflow_mlp_fixed_point': (_i, [_c_fp] * 6 + [_i, _i] + [_c_fp] * 6 + [_i, _f, _f, _i, _c_fp]),
     'impflow_mlp_series': (_i, [_c_fp] * 6 + [_i, _i, _i, _c_fp, _c_fp, _c_fp, _c_fp, _c_fp, _c_fp]),
     'impflow_act_mul': (_i, [_c_fp, _c_fp, _c_fp, _ll, _i, _i, _c_fp, _c_fp]),
     'impflow_act_split': (_i, [_c_fp, _c_fp, _c_fp, _ll, _i, _i, _c_fp, _c_fp]),
@@ -71,6 +72,8 @@ SIGNATURES = {
     'impflow_conv3_set_runahead': (_i, [_i]),
     'impflow_conv3_set_chain_fuse': (_i, [_i]),
     'impflow_conv3_broyden': (_i, [_c_fp, _i] + [_c_fp] * 17 + [_i, _d, _c_fp]),
+    'impflow_conv3_fixed_point_host_bytes': (ctypes.c_size_t, [_i]),
+    'impflow_conv3_fixed_point': (_i, [_c_fp] * 8 + [_f, _f, _i, _c_fp]),
     'impflow_wgrad_set_slice_major': (_i, [_i]),
     'impflow_wgrad_tc_workspace_floats': (ctypes.c_size_t, [_ll, _i, _i]),
     'impflow_wgrad_tc': (_i, [_c_fp, _c_fp, _ll, _c_fp, _c_fp, _ll, _c_fp, _ll, _i, _ll, _i, _i, _c_fp, _c_fp]),

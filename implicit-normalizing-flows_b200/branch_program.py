@@ -86,6 +86,14 @@ def _conv3_workspace(n_floats, device):
     return t
 
 
+def _device_solve(t):
+    """Whether the one-call fixed-point solves take `t`: they drive a CUDA stream (evaluations enqueued ahead of the
+    device's decisions, progress records in mapped pinned memory, one drain per solve), so CUDA tensors only.  A CPU
+    tensor takes the host loop, whose kernel launches refuse it (there is no CPU execution path), as before these
+    solves existed; the numpy C-ABI emulator of the CPU test suite runs that loop."""
+    return t.is_cuda
+
+
 def _round_up(n, m):
     return (n + m - 1) // m * m
 
@@ -672,6 +680,40 @@ class BranchProgram(object):
             info = _broyden.broyden(g, torch.zeros(B, d, device=rows.device), threshold, eps)
         info['result'] = self._from_rows(info['result'].view(M, -1), meta)
         return info
+
+    def fixed_point(self, rhs, start, atol, rtol, threshold):
+        """Banach iteration x_k = rhs - nnet(x_{k-1}) from x_0 = start until every (x_k - x_{k-1})^2 /
+        (atol + |start| rtol) < 1, at most threshold + 2 evaluations (iresblock.py:69-79, implicit_block.py:17-28).
+        Returns (x, the reference's iteration count), x in module layout.
+
+        The whole iteration is one call where the branch allows it: the persistent kernel of a small MLP branch
+        (csrc/mlp_solver.cu), or the native runtime of a 3-layer conv branch (csrc/conv3_plan.cu), which computes what
+        the host loop over forward() computes, bit for bit.  Otherwise (another branch, a CPU tensor, a threshold above
+        the calls' limit of 1000) it is the host loop (find_fixed_point)."""
+        if _device_solve(rhs) and 0 <= threshold <= _broyden.FIXED_POINT_MAX_THRESHOLD:
+            spec = self.mlp_solver_spec(rhs)
+            if spec is not None:
+                return _broyden.fixed_point_mlp(spec, rhs, start, atol, rtol, threshold)
+            P = self.native_plan(rhs)
+            if P is not None:
+                return self._native_fixed_point(P, rhs, start, atol, rtol, threshold)
+        from .layers.implicit_block import find_fixed_point
+        return find_fixed_point(lambda x: ops.lincomb3(rhs, 1.0, self.forward(x), -1.0), start, threshold, atol, rtol)
+
+    def _native_fixed_point(self, P, rhs, start, atol, rtol, threshold):
+        rows, meta = self._to_rows(rhs)
+        srows = rows if start is rhs else self._to_rows(start)[0]
+        ws = _broyden.fixed_point_workspace(rhs.shape[0], rows.numel() // rhs.shape[0], rows.device)
+        out = torch.empty_like(rows)
+        vp = lambda t: ctypes.c_void_p(t.data_ptr())
+        _cabi.check(_cabi.load().impflow_conv3_fixed_point(
+            self._plan_ptr(P), _cabi.ptr(rows), _cabi.ptr(srows), _cabi.ptr(out), _cabi.ptr(ws.xa), _cabi.ptr(ws.xb),
+            vp(ws.state), vp(ws.state_host), float(atol), float(rtol), int(threshold), _cabi.stream()),
+            'conv3_fixed_point')
+        iterations = ws.iterations()
+        if ops.GEMM_PROFILE['on']:
+            self._record_conv3(P, False, False, iterations + 1)
+        return self._from_rows(out, meta).contiguous(), iterations
 
     def _ains(self, saved):
         """Layer-input handles of a saved forward (the fused forward keeps only the pre-activations)."""

@@ -9,6 +9,8 @@
 //   impflow_conv3_broyden        whole forward / implicit-backward root solve: branch evaluations, the
 //                                residual, the solver algebra and the per-iteration state read-back
 //                                (broyden.py:123-193 + implicit_block.py:68-80, 199-207)
+//   impflow_conv3_fixed_point    whole Banach iteration x <- rhs - nnet(x) with its stopping test
+//                                (iresblock.py:69-79, implicit_block.py:17-28)
 //
 // Everything works on NHWC "rows" (M = B*H*W rows of c floats): a sample is a contiguous block of
 // d = H*W*c floats, which is all the solver's per-sample dot products need.  Shapes with 9c <= 32 and
@@ -89,6 +91,8 @@ static int plan_check(const impflow_conv3_plan* p, const char* who) {
 //                   fwd resid: out = (rhs - val) - x           g(z) = x_embed - f(z) - z   (implicit_block.py:72)
 //                   bwd resid: out = (val + x) - rhs           g(v) = v^T J + v - grad     (:199-203)
 //                   chain    : out = val, acc = fma(val, coeff, acc)   w += c_k v^T J^k    (:431-435)
+//                   fixed pt : out = rhs - val, and the element test of the Banach loop against the previous
+//                              iterate x; the last block decides        (iresblock.py:69-79, see fixed_point_decide)
 //                 (the same roundings, in the same order, as the separate lincomb3 launches they replace)
 // Both honour the device gate of the sync-free solver loop (common.cuh).
 // ------------------------------------------------------------------------------------------------------------
@@ -149,7 +153,7 @@ k_conv3_in(const float* __restrict__ x, float* __restrict__ col, float* __restri
   }
 }
 
-enum { OUT_PLAIN = 0, OUT_FWD_RESIDUAL = 1, OUT_BWD_RESIDUAL = 2, OUT_CHAIN = 3 };
+enum { OUT_PLAIN = 0, OUT_FWD_RESIDUAL = 1, OUT_BWD_RESIDUAL = 2, OUT_CHAIN = 3, OUT_FIXED_POINT = 4 };
 
 struct Conv3Out {
   int nparts;           // partial accumulators to sum (chain23: one per 128-channel quarter), fixed order
@@ -173,7 +177,43 @@ struct Conv3Out {
   int next_ld;
   float* zero;          // tap accumulator of the next evaluation to clear (tile kernel), zero_n4 float4 groups
   long long zero_n4;
+  // fixed-point mode: evaluation `iter` of the Banach loop (x = the previous iterate, rhs = the right-hand side)
+  const float* start;   // |start| scales the tolerance (the reference's quirk in the Banach fallback: not |rhs|)
+  impflow_fixed_point_state* fp;
+  BroydenProgress* fp_progress;   // mapped pinned records, index iter - 1
+  float atol, rtol;
+  int iter, threshold;
 };
+
+// Sum of the blocks' failing-element counts (integers: the order of the atomic adds does not matter); the last block
+// to arrive applies the stopping rule of evaluation a.iter, publishes it and re-arms the counters for the next one.
+__device__ __forceinline__ void fixed_point_decide(const Conv3Out& a, int fails) {
+  __shared__ int warp_fails[8];     // 256 threads (launch_out)
+  fails = __reduce_add_sync(0xffffffffu, fails);
+  if ((threadIdx.x & 31) == 0) warp_fails[threadIdx.x >> 5] = fails;
+  __syncthreads();
+  if (threadIdx.x != 0) return;
+  int block = 0;
+  for (int w = 0; w < (int)(blockDim.x >> 5); ++w) block += warp_fails[w];
+  if (block != 0) atomicAdd(&a.fp->fails, block);
+  __threadfence();
+  if (atomicAdd(&a.fp->ticket, 1) != (int)gridDim.x - 1) return;
+  __threadfence();
+  const int total = atomicAdd(&a.fp->fails, 0);
+  const int active = (a.iter - 1 > a.threshold || total == 0) ? 0 : 1;
+  a.fp->iterations = a.iter - 1;
+  a.fp->active = active;
+  a.fp->fails = 0;
+  a.fp->ticket = 0;
+  __threadfence();
+  if (a.fp_progress != nullptr) {
+    volatile BroydenProgress* pr = a.fp_progress + (a.iter - 1);
+    pr->active = active;
+    __threadfence_system();
+    pr->seq = a.iter - 1;
+    __threadfence_system();
+  }
+}
 
 __global__ void __launch_bounds__(256) k_conv3_out(int B, int H, int W, int C, Conv3Out a) {
   pdl_trigger();
@@ -181,6 +221,7 @@ __global__ void __launch_bounds__(256) k_conv3_out(int B, int H, int W, int C, C
   if (gate_closed(a.gate)) return;
   const float beta = (a.beta0 != nullptr) ? __ldg(a.beta0) : 0.f;
   const long long total = (long long)B * H * W * C;
+  int fails = 0;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {
     const int c = (int)(i % C);
@@ -206,7 +247,14 @@ __global__ void __launch_bounds__(256) k_conv3_out(int B, int H, int W, int C, C
       val = sum + (a.bias != nullptr ? a.bias[c] : 0.f);
     }
     float r = val;
-    if (a.mode == OUT_FWD_RESIDUAL) {
+    if (a.mode == OUT_FIXED_POINT) {
+      // x = rhs - f (one rounding, as lincomb3(rhs, 1, f, -1)); test (x - x_prev)^2 / (atol + |start| rtol) < 1 with
+      // the roundings of the torch expression: no contraction into FMAs, a NaN fails
+      r = __fsub_rn(a.rhs[i], val);
+      const float tol = __fadd_rn(a.atol, __fmul_rn(fabsf(a.start[i]), a.rtol));
+      const float dx = __fsub_rn(r, a.x[i]);
+      fails += (__fdiv_rn(__fmul_rn(dx, dx), tol) < 1.f) ? 0 : 1;
+    } else if (a.mode == OUT_FWD_RESIDUAL) {
       r = a.rhs[i] - val;
       r = r - a.x[i];
     } else if (a.mode == OUT_BWD_RESIDUAL) {
@@ -245,6 +293,7 @@ __global__ void __launch_bounds__(256) k_conv3_out(int B, int H, int W, int C, C
          i += (long long)gridDim.x * blockDim.x)
       reinterpret_cast<float4*>(a.zero)[i] = z;
   }
+  if (a.mode == OUT_FIXED_POINT) fixed_point_decide(a, fails);
 }
 
 static inline int grid_cap(long long n, int per) {
@@ -618,4 +667,98 @@ extern "C" int impflow_conv3_broyden(const impflow_conv3_plan* plan, int mode, c
     }
   }
   return read_state();        // full state record (trace, flags) + one stream drain per solve
+}
+
+extern "C" size_t impflow_conv3_fixed_point_host_bytes(int threshold) {
+  return sizeof(impflow_fixed_point_state) + sizeof(BroydenProgress) * (size_t)(threshold + 2);
+}
+
+extern "C" int impflow_conv3_fixed_point(const impflow_conv3_plan* plan, const float* rhs_rows, const float* start_rows,
+                                         float* out_rows, float* xa, float* xb, impflow_fixed_point_state* state_dev,
+                                         impflow_fixed_point_state* state_host, float atol, float rtol, int threshold,
+                                         void* stream) {
+  if (plan_check(plan, "conv3_fixed_point")) return -3;
+  IMPFLOW_REQUIRE(threshold >= 0 && threshold <= 1000, "conv3_fixed_point: threshold %d not in [0,1000]", threshold);
+  const long long M = (long long)plan->B * plan->H * plan->W;
+  const Conv3Ws w = carve(plan->ws, M, plan->c, plan->C, plan->k0);
+  cudaStream_t s = (cudaStream_t)stream;
+  // progress records in mapped pinned memory behind the state record (impflow_conv3_fixed_point_host_bytes), one per
+  // evaluation: record k - 1 is written by the decision of evaluation k
+  BroydenProgress* prog_host = reinterpret_cast<BroydenProgress*>(state_host + 1);
+  BroydenProgress* prog_dev = nullptr;
+  if (cudaHostGetDevicePointer(reinterpret_cast<void**>(&prog_dev), prog_host, 0) != cudaSuccess) {
+    cudaGetLastError();
+    set_error("conv3_fixed_point: state_host is not mapped pinned host memory");
+    return -3;
+  }
+  const int runahead = g_runahead;
+  const int last = threshold + 2;            // evaluations at most
+  float* xs[2] = {xa, xb};                   // evaluation k writes xs[k & 1]: the roles are known ahead
+  auto eval = [&](int k) -> int {
+    const float* prev = k == 1 ? start_rows : xs[(k - 1) & 1];
+    if (conv3_chain_forward(plan, w, prev, nullptr, nullptr, stream)) return -1;
+    Conv3Out a = out_forward(plan, w, xs[k & 1]);
+    a.mode = OUT_FIXED_POINT;
+    a.x = prev;
+    a.rhs = rhs_rows;
+    a.start = start_rows;
+    a.fp = state_dev;
+    a.fp_progress = prog_dev;
+    a.atol = atol;
+    a.rtol = rtol;
+    a.iter = k;
+    a.threshold = threshold;
+    return launch_out(plan, a, s);
+  };
+  volatile BroydenProgress* vp = prog_host;
+  for (int i = 0; i < last; ++i) vp[i].seq = -1;
+  auto wait_for = [&](int rec) -> int {
+    long long spins = 0;
+    while (vp[rec].seq != rec) {
+      if ((++spins & 0x3ff) == 0) {
+        const cudaError_t q = cudaStreamQuery(s);
+        if (q != cudaSuccess && q != cudaErrorNotReady) {
+          set_error("conv3_fixed_point: stream failed while waiting for evaluation %d: %s", rec + 1,
+                    cudaGetErrorString(q));
+          return -1;
+        }
+        if (q == cudaSuccess && vp[rec].seq != rec) {
+          set_error("conv3_fixed_point: evaluation %d never reported (stream idle)", rec + 1);
+          return -1;
+        }
+      }
+    }
+    return 0;
+  };
+  // zero counters and ticket; evaluation 1 always runs (ungated), its decision opens or closes the gate
+  if (cudaMemsetAsync(state_dev, 0, sizeof(impflow_fixed_point_state), s) != cudaSuccess) {
+    set_error("conv3_fixed_point: state reset failed");
+    return -1;
+  }
+  {
+    GateScope ungated(nullptr);
+    if (eval(1)) return -1;
+  }
+  int seen = 0, enq = 1;       // decisions seen / evaluations enqueued
+  {
+    GateScope gated(&state_dev->active);
+    for (;;) {
+      while (enq < seen + 1 + runahead && enq < last) {
+        if (eval(++enq)) return -1;
+      }
+      if (wait_for(seen)) return -1;
+      ++seen;
+      if (!vp[seen - 1].active) break;
+    }
+  }
+  // evaluation `seen` ended the loop; the gated evaluations behind it wrote nothing
+  const size_t bytes = sizeof(float) * (size_t)M * plan->c;
+  if (cudaMemcpyAsync(out_rows, xs[seen & 1], bytes, cudaMemcpyDeviceToDevice, s) != cudaSuccess ||
+      cudaMemcpyAsync(state_host, state_dev, sizeof(impflow_fixed_point_state), cudaMemcpyDeviceToHost, s) !=
+          cudaSuccess ||
+      cudaStreamSynchronize(s) != cudaSuccess) {
+    set_error("conv3_fixed_point: result copy failed: %s", cudaGetErrorString(cudaGetLastError()));
+    return -1;
+  }
+  return 0;
 }

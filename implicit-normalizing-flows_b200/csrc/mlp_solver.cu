@@ -317,6 +317,83 @@ k_mlp_broyden(MlpDesc net, const float* __restrict__ x_embed, float* za, float* 
 
 
 // ------------------------------------------------------------------------------------------------------------
+// Banach fixed-point iteration of the same branches in ONE cooperative launch (iresblock.py:69-79,
+// implicit_block.py:17-28; the contract is in the header at impflow_conv3_fixed_point):
+//     x_k = rhs - f(x_{k-1}),  x_0 = start,  stop when k - 1 > T or every (x_k - x_{k-1})^2 / (atol + |start| rtol) < 1.
+// A CTA owns its tiles for the whole solve (it reads only the iterates it wrote), so the one grid.sync per evaluation
+// is for the failing-element counts alone.  They are integers, summed by every CTA in the same way, so every CTA takes
+// the same decision.  The counts are double-buffered by the parity of k: a CTA that is already in evaluation k + 1
+// writes the other half while a slower one still reads the counts of evaluation k.
+// ------------------------------------------------------------------------------------------------------------
+// (3 CTAs per SM: without the hint ptxas keeps 40 registers and spills around the mlp_eval calls)
+__global__ void __launch_bounds__(kMlpThreads, 3)
+k_mlp_fixed_point(MlpDesc net, const float* __restrict__ rhs, const float* __restrict__ start, float* __restrict__ out,
+                  float* xa, float* xb, int* __restrict__ counts, impflow_fixed_point_state* state, int B, float atol,
+                  float rtol, int T) {
+  cg::grid_group grid = cg::this_grid();
+  __shared__ __align__(16) float bufA[kTile * kMaxWidth];
+  __shared__ __align__(16) float bufB[kTile * kMaxWidth];
+  __shared__ int red[kMlpWarps];
+  const int d = net.dims[0];
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  const int n_tiles = (B + kTile - 1) / kTile;
+  int k = 1;
+  for (;; ++k) {
+    float* cur = (k & 1) ? xb : xa;                                 // evaluation k writes xa (k even) / xb (k odd)
+    const float* prev = k == 1 ? start : ((k & 1) ? xa : xb);       // and reads what evaluation k - 1 wrote
+    int fails = 0;
+    for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+      const int s0 = tile * kTile;
+      const float* f = mlp_eval(net, prev, s0, B, bufA, bufB);
+      for (int i = tid; i < kTile * d; i += kMlpThreads) {
+        const int s = i / d, c = i % d;
+        if (s0 + s >= B) continue;
+        const long long idx = (long long)(s0 + s) * d + c;
+        // one rounding per operation, as the torch expression of the reference loop
+        const float x = __fsub_rn(rhs[idx], f[s * kMaxWidth + c]);
+        const float tol = __fadd_rn(atol, __fmul_rn(fabsf(start[idx]), rtol));
+        const float dx = __fsub_rn(x, prev[idx]);
+        fails += (__fdiv_rn(__fmul_rn(dx, dx), tol) < 1.f) ? 0 : 1;
+        cur[idx] = x;
+      }
+      __syncthreads();      // bufA / bufB are reused by the next tile
+    }
+    fails = __reduce_add_sync(0xffffffffu, fails);
+    if (lane == 0) red[warp] = fails;
+    __syncthreads();
+    if (tid == 0) {
+      int t = 0;
+      for (int w = 0; w < kMlpWarps; ++w) t += red[w];
+      counts[(k & 1) * gridDim.x + blockIdx.x] = t;
+    }
+    grid.sync();
+    int total = 0;
+    for (int i = tid; i < (int)gridDim.x; i += kMlpThreads) total += __ldcg(&counts[(k & 1) * gridDim.x + i]);
+    total = __reduce_add_sync(0xffffffffu, total);
+    __syncthreads();      // every warp has read red[] above before it is overwritten
+    if (lane == 0) red[warp] = total;
+    __syncthreads();
+    total = 0;
+    for (int w = 0; w < kMlpWarps; ++w) total += red[w];
+    __syncthreads();      // red[] is reused by the next evaluation
+    if (k - 1 > T || total == 0) break;
+  }
+  // the final iterate of this CTA's tiles into the caller's buffer
+  const float* fin = (k & 1) ? xb : xa;
+  for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x)
+    for (int i = tid; i < kTile * d; i += kMlpThreads) {
+      const long long idx = (long long)tile * kTile * d + i;
+      if (idx < (long long)B * d) out[idx] = fin[idx];
+    }
+  if (blockIdx.x == 0 && tid == 0) {
+    state->iterations = k - 1;
+    state->active = 0;
+    state->fails = 0;
+    state->ticket = 0;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------------------
 // Power series of a small-d MLP branch in ONE launch (north-star kernel (c) for the MLP flows): the training path of
 // the basic estimator (implicit_block.py:418-426 with create_graph=True) needs, at one saved point and for one probe v,
 //     left vectors   l_k = (J^T)^k v, k = 1..n      (vjp chain)          S = sum_k c_k <l_k, v>
@@ -401,6 +478,7 @@ k_mlp_series(MlpDesc vjp, MlpDesc tan, SeriesCoeffs co, const float* __restrict_
 }  // namespace impflow
 
 namespace impflow {
+int mlp_cooperative_grid(const void* kernel, int B, int* grid);
 int launch_mlp_solver(MlpDesc net, const float* x_embed, float* za, float* ga, float* zb, float* gb, float* low_z,
                       float* low_g, float* Ut, float* Vt, float* sample_sq, float* low_sq, double* partial,
                       impflow_broyden_state* state, int B, int threshold, double eps_scaled, void* stream);
@@ -491,18 +569,8 @@ namespace impflow {
 int launch_mlp_solver(MlpDesc net, const float* x_embed, float* za, float* ga, float* zb, float* gb, float* low_z,
                       float* low_g, float* Ut, float* Vt, float* sample_sq, float* low_sq, double* partial,
                       impflow_broyden_state* state, int B, int threshold, double eps_scaled, void* stream) {
-  int dev = 0, sms = 0, per_sm = 0;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_mlp_broyden, kMlpThreads, 0) != cudaSuccess ||
-      per_sm < 1) {
-    set_error("mlp_broyden_solve: occupancy query failed");
-    return -1;
-  }
-  const int n_tiles = (B + kTile - 1) / kTile;
-  int grid = sms * (per_sm > 8 ? 8 : per_sm);
-  if (grid > n_tiles) grid = n_tiles;
-  if (grid > 148 * 8) grid = 148 * 8;
+  int grid = 0;
+  if (mlp_cooperative_grid((const void*)k_mlp_broyden, B, &grid)) return -1;
   int T = threshold;
   double eps = eps_scaled;
   void* args[] = {&net, &x_embed, &za, &ga, &zb, &gb, &low_z, &low_g, &Ut, &Vt, &sample_sq, &low_sq,
@@ -515,7 +583,74 @@ int launch_mlp_solver(MlpDesc net, const float* x_embed, float* za, float* ga, f
   }
   return check_launch("k_mlp_broyden");
 }
+
+// Grid of a persistent cooperative kernel: every CTA resident (up to 8 per SM), no more CTAs than tiles, at most
+// 148 * 8 (the size of the per-CTA partial buffers).
+int mlp_cooperative_grid(const void* kernel, int B, int* grid) {
+  int dev = 0, sms = 0, per_sm = 0;
+  cudaGetDevice(&dev);
+  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kMlpThreads, 0) != cudaSuccess || per_sm < 1) {
+    set_error("mlp solver: occupancy query failed");
+    return -1;
+  }
+  const int n_tiles = (B + kTile - 1) / kTile;
+  int g = sms * (per_sm > 8 ? 8 : per_sm);
+  if (g > n_tiles) g = n_tiles;
+  if (g > 148 * 8) g = 148 * 8;
+  *grid = g;
+  return 0;
+}
 }  // namespace impflow
+
+extern "C" int impflow_mlp_fixed_point(const float* rhs, const float* start, float* out, const float* const* Wt,
+                                       const float* const* bias, const int* dims, int L, int act_kind,
+                                       const float* const* beta_sp, float* xa, float* xb, int* counts,
+                                       impflow_fixed_point_state* state_dev, impflow_fixed_point_state* state_host,
+                                       int B, float atol, float rtol, int threshold, void* stream) {
+  IMPFLOW_REQUIRE(L >= 1 && L <= kMaxLayers, "mlp_fixed_point: %d layers not in [1,%d]", L, kMaxLayers);
+  IMPFLOW_REQUIRE(threshold >= 0 && threshold <= 1000, "mlp_fixed_point: threshold %d not in [0,1000]", threshold);
+  IMPFLOW_REQUIRE(dims[0] == dims[L] && dims[0] <= 128, "mlp_fixed_point: needs d_in == d_out <= 128");
+  IMPFLOW_REQUIRE(B >= 1, "mlp_fixed_point: empty batch");
+  IMPFLOW_REQUIRE(act_kind != IMPFLOW_ACT_LIPSWISH || beta_sp != nullptr, "mlp_fixed_point: LipSwish needs beta");
+  if (act_kind == IMPFLOW_ACT_LIPSWISH)
+    for (int l = 0; l + 1 < L; ++l)
+      IMPFLOW_REQUIRE(beta_sp[l] != nullptr, "mlp_fixed_point: LipSwish behind layer %d has no beta", l);
+  MlpDesc net;
+  memset(&net, 0, sizeof(net));
+  net.L = L;
+  for (int l = 0; l <= L; ++l) {
+    IMPFLOW_REQUIRE(dims[l] >= 1 && dims[l] <= kMaxWidth, "mlp_fixed_point: width %d not in [1,%d]", dims[l],
+                    kMaxWidth);
+    net.dims[l] = dims[l];
+  }
+  for (int l = 0; l < L; ++l) {
+    net.Wt[l] = Wt[l];
+    net.ld[l] = dims[l + 1];
+    net.bias[l] = bias ? bias[l] : nullptr;
+  }
+  net.act_kind = act_kind;
+  for (int l = 0; l + 1 < L; ++l) net.beta[l] = beta_sp != nullptr ? beta_sp[l] : nullptr;
+  net.mode = 0;
+  int grid = 0;
+  if (mlp_cooperative_grid((const void*)k_mlp_fixed_point, B, &grid)) return -1;
+  int T = threshold;
+  void* args[] = {&net, &rhs, &start, &out, &xa, &xb, &counts, &state_dev, &B, &atol, &rtol, &T};
+  cudaStream_t s = (cudaStream_t)stream;
+  const cudaError_t e = cudaLaunchCooperativeKernel((void*)k_mlp_fixed_point, dim3(grid), dim3(kMlpThreads), args, 0, s);
+  if (e != cudaSuccess) {
+    set_error("mlp_fixed_point: cooperative launch failed: %s", cudaGetErrorString(e));
+    return -1;
+  }
+  if (check_launch("k_mlp_fixed_point")) return -1;
+  if (cudaMemcpyAsync(state_host, state_dev, sizeof(impflow_fixed_point_state), cudaMemcpyDeviceToHost, s) !=
+          cudaSuccess ||
+      cudaStreamSynchronize(s) != cudaSuccess) {
+    set_error("mlp_fixed_point: state read-back failed: %s", cudaGetErrorString(cudaGetLastError()));
+    return -1;
+  }
+  return 0;
+}
 
 /* One-launch power series of a small-d MLP branch at a saved point (see k_mlp_series):
  *   W[l], ldw[l] : effective weight of layer l, [dims[l+1]][ldw[l]] row-major (vjp chain, as in ..._solve_vjp)

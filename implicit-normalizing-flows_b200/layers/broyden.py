@@ -12,7 +12,7 @@ import torch
 
 from .. import _cabi
 
-__all__ = ['broyden_mlp_vjp', 'broyden', 'broyden_mlp']
+__all__ = ['broyden_mlp_vjp', 'broyden', 'broyden_mlp', 'fixed_point_mlp']
 
 _STATE_DTYPE = np.dtype([('nstep', '<i4'), ('lowest_step', '<i4'), ('active', '<i4'), ('prot_break', '<i4'),
                          ('converged', '<i4'), ('stagnated', '<i4'), ('do_update', '<i4'), ('new_lowest', '<i4'),
@@ -74,6 +74,47 @@ def _workspace(B, d, T, device):
     return ws
 
 
+_FP_STATE_DTYPE = np.dtype([('iterations', '<i4'), ('active', '<i4'), ('fails', '<i4'), ('ticket', '<i4')])
+FIXED_POINT_MAX_THRESHOLD = 1000        # the one-call fixed-point solves' ABI limit
+_fp_workspaces = {}
+
+
+class _FixedPointWorkspace(object):
+    """Buffers of the one-call fixed-point solves (impflow_conv3_fixed_point / impflow_mlp_fixed_point) of one (B, d)
+    size: the two iterates, the device state record, its pinned host copy followed by the conv solve's progress
+    records, and the MLP kernel's per-CTA counts (on first use)."""
+
+    def __init__(self, B, d, device):
+        lib = _cabi.load()
+        f32 = dict(device=device, dtype=torch.float32)
+        self.xa = torch.empty(B, d, **f32)
+        self.xb = torch.empty(B, d, **f32)
+        self.state = torch.zeros(_FP_STATE_DTYPE.itemsize, device=device, dtype=torch.uint8)
+        self.state_host = _cabi.pinned_bytes(int(lib.impflow_conv3_fixed_point_host_bytes(FIXED_POINT_MAX_THRESHOLD)))
+        self.counts = None
+
+    def mlp_counts(self):
+        if self.counts is None:
+            n = 2 * int(_cabi.load().impflow_mlp_solver_partial_doubles())
+            self.counts = torch.empty(n, device=self.xa.device, dtype=torch.int32)
+        return self.counts
+
+    def iterations(self):
+        return int(self.state_host[:_FP_STATE_DTYPE.itemsize].numpy().view(_FP_STATE_DTYPE)[0]['iterations'])
+
+
+def fixed_point_workspace(B, d, device):
+    """The fixed-point workspace of (B, d) on the current stream, cached like _workspace.  A solve drains its stream
+    before it returns, so back-to-back solves may share one; solves on different streams get their own."""
+    key = (B, d, device.index, getattr(_cabi.stream(), 'value', None))
+    ws = _fp_workspaces.get(key)
+    if ws is None:
+        if len(_fp_workspaces) > 16:
+            _fp_workspaces.clear()
+        ws = _fp_workspaces[key] = _FixedPointWorkspace(B, d, device)
+    return ws
+
+
 def scaled_eps(eps, B, d):
     """The stopping tolerance of a solve on the norm of the whole (B, d) residual (broyden.py:131)."""
     return eps * math.sqrt(B * d)
@@ -111,13 +152,7 @@ def broyden_mlp(spec, x_embed, z0, threshold, eps):
     ws.one_call_buffers(mlp=True)
     ws.xa.copy_(z0.reshape(B, d))
     L = len(Wt)
-    wt_arr = (ctypes.c_void_p * L)(*[w.data_ptr() for w in Wt])
-    b_arr = (ctypes.c_void_p * L)(*[(b.data_ptr() if b is not None else None) for b in bias])
-    dims_arr = (ctypes.c_int * (L + 1))(*dims)
-    # one device scalar per activation: every Swish module owns its own learnable beta (activations.py:64-71)
-    beta_arr = None
-    if beta_sp is not None:
-        beta_arr = (ctypes.c_void_p * L)(*([_cabi.ptr(b, 'beta') for b in beta_sp] + [None] * (L - len(beta_sp))))
+    wt_arr, b_arr, dims_arr, beta_arr = _mlp_arrays(Wt, bias, dims, beta_sp)
     xe = x_embed.reshape(B, d).contiguous()
     _cabi.check(lib.impflow_mlp_broyden_solve(
         _cabi.ptr(xe), wt_arr, b_arr, dims_arr, L, act_kind, beta_arr, _cabi.ptr(ws.xa),
@@ -158,6 +193,41 @@ def broyden_mlp_vjp(spec, rhs, threshold, eps):
         ctypes.c_void_p(ws.state.data_ptr()), B, threshold, float(eps_scaled), _cabi.stream()), 'mlp_broyden_solve_vjp')
     state = ws.read_state()
     return _result_dict(ws, state, shape, eps_scaled, threshold)
+
+
+def _mlp_arrays(Wt, bias, dims, beta_sp):
+    """ctypes arrays of the persistent kernels' forward-mode weight description (BranchProgram.mlp_solver_spec)."""
+    L = len(Wt)
+    wt_arr = (ctypes.c_void_p * L)(*[w.data_ptr() for w in Wt])
+    b_arr = (ctypes.c_void_p * L)(*[(b.data_ptr() if b is not None else None) for b in bias])
+    dims_arr = (ctypes.c_int * (L + 1))(*dims)
+    # one device scalar per activation: every Swish module owns its own learnable beta (activations.py:64-71)
+    beta_arr = None
+    if beta_sp is not None:
+        beta_arr = (ctypes.c_void_p * L)(*([_cabi.ptr(b, 'beta') for b in beta_sp] + [None] * (L - len(beta_sp))))
+    return wt_arr, b_arr, dims_arr, beta_arr
+
+
+def fixed_point_mlp(spec, rhs, start, atol, rtol, threshold):
+    """Banach iteration x <- rhs - f(x) from `start` (iresblock.py:69-79, implicit_block.py:17-28) in ONE persistent
+    cooperative kernel (csrc/mlp_solver.cu: k_mlp_fixed_point) for the MLP branches `spec` describes
+    (BranchProgram.mlp_solver_spec).  Returns (x shaped like rhs, the reference's iteration count)."""
+    _cabi.require_device(rhs, 'fixed_point_mlp rhs')
+    lib = _cabi.load()
+    Wt, bias, dims, act_kind, beta_sp = spec
+    d = dims[0]
+    r = rhs.reshape(-1, d).contiguous()
+    s = start.reshape(-1, d).contiguous()
+    B = r.shape[0]
+    ws = fixed_point_workspace(B, d, r.device)
+    out = torch.empty_like(r)
+    wt_arr, b_arr, dims_arr, beta_arr = _mlp_arrays(Wt, bias, dims, beta_sp)
+    _cabi.check(lib.impflow_mlp_fixed_point(
+        _cabi.ptr(r), _cabi.ptr(s), _cabi.ptr(out), wt_arr, b_arr, dims_arr, len(Wt), act_kind, beta_arr,
+        _cabi.ptr(ws.xa), _cabi.ptr(ws.xb), ctypes.c_void_p(ws.mlp_counts().data_ptr()),
+        ctypes.c_void_p(ws.state.data_ptr()), ctypes.c_void_p(ws.state_host.data_ptr()), B, float(atol), float(rtol),
+        int(threshold), _cabi.stream()), 'mlp_fixed_point')
+    return out.view(rhs.shape), ws.iterations()
 
 
 def broyden(g_, x0, threshold, eps, ls=False, name='unknown'):

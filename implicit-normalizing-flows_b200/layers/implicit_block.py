@@ -220,17 +220,35 @@ def _upload(host_t, like):
     return buf.to(like.device, non_blocking=True).view(host_t.shape)
 
 
-def find_fixed_point(g, y, threshold=1000, eps=1e-5):
-    """Banach iteration, fallback after a protective break (implicit_block.py:17-28)."""
+def find_fixed_point(g, y, threshold=1000, atol=1e-5, rtol=1e-5):
+    """Banach iteration x <- g(x) from y on the host (implicit_block.py:17-28, iresblock.py:69-79): until every
+    (x - x_prev)^2 / (atol + |y| rtol) < 1, at most threshold + 2 evaluations of g.  Returns (x, i), i the reference's
+    iteration count.  Builds a graph through g when grad mode is on."""
     x, x_prev = g(y), y
     i = 0
-    tol = eps + eps * y.abs()
+    tol = atol + y.abs() * rtol
     while not torch.all((x - x_prev) ** 2 / tol < 1.):
         x, x_prev = g(x), x
         i += 1
         if i > threshold:
             break
-    return x
+    return x, i
+
+
+def solve_fixed_point(nnet, rhs, start, atol, rtol, threshold=1000):
+    """x = rhs - nnet(x) by Banach iteration from x = start, the tolerance scaled by |start|: (x, iterations).
+    iResBlock's inverse has rhs = start = y (iresblock.py:69-79); the Banach fallback of RootFind has rhs = x_embed,
+    start = z0 (implicit_block.py:17-28, 74-75).  Without a graph, a compiled branch runs BranchProgram.fixed_point
+    (one call per solve where the branch allows it); otherwise the host loop goes through the module, building the
+    graph when one is needed."""
+    graph_free = not (torch.is_grad_enabled() and (rhs.requires_grad or start.requires_grad
+                                                   or any(p.requires_grad for p in nnet.parameters())))
+    prog = _program(nnet) if graph_free else None
+    if prog is not None:
+        with torch.no_grad():
+            return prog.fixed_point(rhs, start, atol, rtol, threshold)
+    with torch.set_grad_enabled(not graph_free):
+        return find_fixed_point(lambda x: rhs - nnet(x), start, threshold, atol, rtol)
 
 
 class RootFind(Function):
@@ -245,7 +263,7 @@ class RootFind(Function):
     def banach_find_root(nnet_z, nnet_x, z0, x, *args):
         eps, threshold = args[-2], args[-1]
         x_embed = branch_eval(nnet_x, x) + x
-        z_est = find_fixed_point(lambda z: x_embed - branch_eval(nnet_z, z), z0, threshold=threshold, eps=eps)
+        z_est, _ = solve_fixed_point(nnet_z, x_embed, z0, eps, eps, threshold)
         return z_est.clone().detach()
 
     @staticmethod

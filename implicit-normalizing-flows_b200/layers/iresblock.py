@@ -11,7 +11,8 @@ What runs where (shared with imBlock, see implicit_block.py):
     also returns g and back-propagates grad_g through the kept graph; here g is the output of the branch
     program's own autograd node, so autograd adds the two contributions;
   * eval-mode log-det (20 exact terms): the vjp chain on the fused kernels with in-place Hutchinson dots;
-  * inverse: Banach iteration x <- y - g(x) (:69-79) on the fused forward, convergence test as in the reference.
+  * inverse: Banach iteration x <- y - g(x) (:69-79), convergence test as in the reference: one call per solve on
+    the native conv runtime or the persistent MLP kernel where the branch allows it (BranchProgram.fixed_point).
 Gaussian probes are drawn with randn_like on the device like the reference does (:129); tests inject them.
 
 `forward` additionally accepts (and ignores) `restore=`: SequentialFlow passes it to every layer, which makes
@@ -20,7 +21,6 @@ import numpy as np
 import torch
 import torch.nn as nn
 
-from .. import ops
 from . import implicit_block as ib
 
 __all__ = ['iResBlock']
@@ -64,22 +64,7 @@ class iResBlock(nn.Module):
 
     def _inverse_fixed_point(self, y, atol=1e-5, rtol=1e-5):
         """x <- y - g(x) until every (x - x_prev)^2 / (atol + rtol |y|) < 1, cap 1000 (iresblock.py:69-79)."""
-        graph_free = not (torch.is_grad_enabled() and (y.requires_grad or any(p.requires_grad
-                                                                               for p in self.nnet.parameters())))
-        if graph_free and ib._program(self.nnet) is not None:
-            step = lambda x: ops.lincomb3(y, 1.0, ib.branch_eval(self.nnet, x), -1.0)
-        else:
-            step = lambda x: y - self.nnet(x)
-        with torch.set_grad_enabled(not graph_free):
-            x, x_prev = step(y), y
-            i = 0
-            tol = atol + y.abs() * rtol
-            while not torch.all((x - x_prev) ** 2 / tol < 1):
-                x, x_prev = step(x), x
-                i += 1
-                if i > 1000:
-                    break
-        self.inverse_iterations = i
+        x, self.inverse_iterations = ib.solve_fixed_point(self.nnet, y, y, atol, rtol, 1000)
         return x
 
     # --------------------------------------------------------------------------------------

@@ -388,6 +388,47 @@ int impflow_conv3_broyden(const impflow_conv3_plan* plan, int mode, const float*
                           double eps_scaled, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * Banach fixed-point iteration — replaces the host loops of iresblock.py:69-79 (iResBlock inverse) and
+ * implicit_block.py:17-28 (find_fixed_point, the fallback after a protective Broyden break):
+ *     x_k = rhs - nnet(x_{k-1}),  x_0 = start,
+ * stopping after evaluation k when k - 1 > threshold (no test), or when every element satisfies
+ * (x_k - x_{k-1})^2 / (atol + |start| * rtol) < 1, each operation rounded once as the torch expression rounds it (a
+ * NaN fails the test).  The reported count is the reference's i = k - 1, so there are at most threshold + 2
+ * evaluations; 0 <= threshold <= 1000.  The test is batch-global (torch.all over the whole tensor).
+ * These entry points were added without an ABI version change: no existing signature or struct changed.
+ * ------------------------------------------------------------------------------------------ */
+typedef struct {
+  int32_t iterations;   /* the reference's count i (iResBlock.inverse_iterations) once the loop has ended */
+  int32_t active;       /* 1 while the loop continues */
+  int32_t fails;        /* internal: elements of the current evaluation that fail the test */
+  int32_t ticket;       /* internal: last-block election */
+} impflow_fixed_point_state;
+
+/* Conv branch, rows layout, one call per solve: per evaluation the branch's kernels, then the col2im epilogue writes
+ * x_k = rhs - f and counts the failing elements, and its last block takes the decision.  Iterates alternate between
+ * xa and xb ((M, c) scratch each); the host enqueues up to `runahead` evaluations (impflow_conv3_set_runahead) past
+ * the last decision it has seen, behind the same device-side gate as impflow_conv3_broyden, and learns the decisions
+ * from progress records in mapped pinned memory.  At the end the final iterate is copied into out_rows and the
+ * stream is drained once.
+ * state_host: PINNED host memory of impflow_conv3_fixed_point_host_bytes(threshold) bytes; on return it starts with
+ * the final state record. */
+size_t impflow_conv3_fixed_point_host_bytes(int threshold);
+int impflow_conv3_fixed_point(const impflow_conv3_plan* plan, const float* rhs_rows, const float* start_rows,
+                              float* out_rows, float* xa, float* xb, impflow_fixed_point_state* state_dev,
+                              impflow_fixed_point_state* state_host, float atol, float rtol, int threshold,
+                              void* stream);
+/* Small MLP branch (the branches impflow_mlp_broyden_solve takes, same Wt / bias / dims / act_kind / beta_sp): the
+ * whole iteration in ONE cooperative launch, one grid-wide barrier per evaluation.  rhs / start / out are (B, d);
+ * xa / xb are (B, d) scratch; counts is an int workspace of 2 * impflow_mlp_solver_partial_doubles() ints (the
+ * persistent solver's `partial` buffer holds that many).  The final state record is copied into state_host (host
+ * memory, pinned for an asynchronous copy) and the stream is drained once. */
+int impflow_mlp_fixed_point(const float* rhs, const float* start, float* out, const float* const* Wt,
+                            const float* const* bias, const int* dims, int L, int act_kind,
+                            const float* const* beta_sp, float* xa, float* xb, int* counts,
+                            impflow_fixed_point_state* state_dev, impflow_fixed_point_state* state_host, int B,
+                            float atol, float rtol, int threshold, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Induced 2-norm power iteration for a dense (out,in) matrix — replaces
  * mixed_lipschitz.py:85-123 (Linear) and :276-319 (1x1 conv).  One CTA, device-side early
  * exit with the reference tolerance rule; u, v updated in place; sigma[0] = u^T W v,
