@@ -87,6 +87,11 @@ SIGNATURES = {
     'impflow_sn_scale': (_i, [_c_fp, _c_fp, _f, _c_fp, _c_fp, _ll, _c_fp]),
     'impflow_sn_scale_grad': (_i, [_c_fp, _c_fp, _c_fp, _c_fp, _f, _c_fp, _ll, _c_fp]),
     'impflow_sn_scale_grad_layout': (_i, [_c_fp, _ll, _c_fp, _c_fp, _c_fp, _f, _i, _i, _i, _c_fp, _c_fp, _c_fp]),
+    'impflow_prep_weights_lop': (_i, [_c_fp, _c_fp, _i, _f, _i, _i, _i, _c_fp, _c_fp, _c_fp, _i, _i, _c_fp, _c_fp,
+                                      _c_fp, _i, _i, _c_fp]),
+    'impflow_lop_norms': (_i, [_c_fp, _i, _i, _i, _i, _i, _c_fp, _c_fp, _c_fp]),
+    'impflow_lop_scale_grad_layout': (_i, [_c_fp, _ll, _c_fp, _c_fp, _f, _i, _i, _i, _i, _i, _i, _c_fp, _c_fp,
+                                           _c_fp]),
     'impflow_sn_conv_set_ctas': (_i, [_i]),
     'impflow_sn_conv_workspace_floats': (ctypes.c_size_t, [_i, _i, _i, _i]),
     'impflow_sn_power_iter_conv3x3': (_i, [_c_fp] * 5 + [_i, _i, _i, _i, _i, _f, _f, _c_fp, _c_fp, _c_fp]),

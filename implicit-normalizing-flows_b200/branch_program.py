@@ -7,8 +7,8 @@ vjps, the n-term vjp chain of the power series, the estimator's double backward)
 one of them through nn.Module.__call__ + autograd costs thousands of tiny launches; the arithmetic
 is a handful of GEMMs.  A BranchProgram compiles an nn.Sequential of
     [act] layer act layer ... layer [act]
-(InducedNormLinear / InducedNormConv2d 1x1 / 3x3 + Sin / Swish / ReLU: every branch the shipped
-configs build — train_toy.py:146-171, train_tabular.py:292-311, implicit_flow.py:359-398,
+(InducedNormLinear / InducedNormConv2d and LopLinear / LopConv2d, 1x1 / 3x3, + Sin / Swish / ReLU: every branch the
+shipped configs build — train_toy.py:146-171, train_tabular.py:292-311, implicit_flow.py:359-398,
 train_classification.py:152-167) into:
 
   forward(x)            nnet(x)                                      (implicit_block.py:68-80)
@@ -20,8 +20,8 @@ Layer forms (rows = pixels or samples, channels contiguous):
   mm   : linear / 1x1 conv          y = A W^T
   c3 A : 3x3, cin <= cout           y = im2col(A) Wr^T        transpose: col2im(G W2t^T)
   c3 B : 3x3, cin >  cout           y = col2im(A W2^T)        transpose: im2col(G) Wrt^T
-The spectrally rescaled weights (compute_weight(update=False)), their GEMM re-layouts and tf32
-hi/lo planes are cached until a parameter / u / v / beta changes version.
+The rescaled weights (compute_weight(update=False) of an induced-norm layer, compute_weight() of a Lop layer), their GEMM
+re-layouts and tf32 hi/lo planes are cached until a parameter / u / v / beta changes version.
 
 neumann() differentiates S = sum_b <w_b, J_b v_b> by hand: S is the forward-mode tangent of the
 branch in direction v contracted with w, so one tangent sweep (t_{l} = W phi'(p) t_{l-1}) plus one
@@ -41,6 +41,7 @@ import torch.nn.functional as F
 from . import _cabi, ops
 from .layers import broyden as _broyden
 from .layers.base.activations import ReLU, Sin, Swish
+from .layers.base.lipschitz import LopConv2d, LopLinear
 from .layers.base.mixed_lipschitz import InducedNormConv2d, InducedNormLinear, sigma_of
 
 __all__ = ['BranchProgram', 'compile_branch', 'FUSED3', 'CONV3_NATIVE', 'MEMO', 'SWEEP_GRAPHS', 'MLP_SERIES']
@@ -75,6 +76,8 @@ TC_MIN_FLOPS = {'program': 2.5e8}      # smallest GEMM a branch program sends to
 MLP_SERIES = {'on': True}      # one-launch vjp / tangent chains of the basic estimator's training path (MLP branches)
 SWEEP_GRAPHS = {'on': True, 'max_rows': 16384, 'warmup': 1, 'mlp': True}
 
+_LINEAR = (InducedNormLinear, LopLinear)          # layers of the linear kind; the others are convolutions
+_LOP = (LopLinear, LopConv2d)                       # closed-form operator-norm layers (rescaled by group norms)
 _conv3_ws = {}      # (device index, stream) -> workspace tensor shared by every plan used on that stream
 
 
@@ -92,6 +95,13 @@ def _device_solve(t):
     tensor takes the host loop, whose kernel launches refuse it (there is no CPU execution path), as before these
     solves existed; the numpy C-ABI emulator of the CPU test suite runs that loop."""
     return t.is_cuda
+
+
+def _device_lop(w):
+    """Whether a branch with Lop layers whose weight is `w` compiles to a program: the Lop weight preparation and
+    gradient chain are CUDA kernels, so CUDA weights only.  A branch on the CPU keeps the module path, as before these
+    kernels existed (the product has no CPU execution path; the numpy C-ABI emulator of the CPU test suite runs it)."""
+    return w.is_cuda
 
 
 def _round_up(n, m):
@@ -123,7 +133,7 @@ _MULT = _Act(ops.ACT_MULTIPLIER)
 class _Weights(object):
     """Effective weights of one layer in the layouts the fused path needs (fp32 + optional planes)."""
     __slots__ = ('fwd', 'fwd_split', 'bwd', 'bwd_split', 'bias', 'kind', 'cin', 'cout', 'fwd_k', 'bwd_k', 'a_type',
-                 'sigma')
+                 'sigma', 'src', 'norms')     # sigma: induced-norm layers; src (raw W) and norms: Lop layers
 
 
 class _T(object):
@@ -175,14 +185,16 @@ def compile_branch(nnet):
             if pending is not None:
                 return None
             pending = a
-        elif isinstance(m, (InducedNormLinear, InducedNormConv2d)):
+        elif isinstance(m, (InducedNormLinear, InducedNormConv2d) + _LOP):
             stages.append((pending, m))
             pending = None
         else:
             return None
     if not stages:
         return None
-    kinds = {isinstance(m, InducedNormLinear) for _, m in stages}
+    if any(isinstance(m, _LOP) for _, m in stages) and not _device_lop(stages[0][1].weight):
+        return None
+    kinds = {isinstance(m, _LINEAR) for _, m in stages}
     if len(kinds) != 1:
         return None
     return BranchProgram(stages, pending, flatten, list(nnet.parameters()))
@@ -195,7 +207,7 @@ class BranchProgram(object):
         self.post_act = post_act
         self.flatten = flatten
         self.params = params            # nnet.parameters() order: the order gradients are returned in
-        self.is_linear = isinstance(stages[0][1], InducedNormLinear)
+        self.is_linear = isinstance(stages[0][1], _LINEAR)
         self._key = None
         self._weights = None
         self._saved = None
@@ -211,8 +223,9 @@ class BranchProgram(object):
     def _version_key(self):
         key = []
         for act, m in self.stages:
-            key += [m.weight._version, m.u._version, m.v._version, m.weight.data_ptr(),
-                    (m.bias._version if m.bias is not None else -1)]
+            key += [m.weight._version, m.weight.data_ptr(), (m.bias._version if m.bias is not None else -1)]
+            if not isinstance(m, _LOP):
+                key += [m.u._version, m.v._version]
         for act in self._acts():
             if act is not None and act.module is not None:
                 key += [act.module.beta._version, act.module.beta.data_ptr()]
@@ -254,12 +267,17 @@ class BranchProgram(object):
                     m._hw = None
                 if isinstance(m, InducedNormConv2d) and not m.is_initialized():
                     m.compute_weight(update=False)                      # lazy u/v init (first use only)
-                # effective weight W / max(1, sigma/coeff) in every layout the kernels consume: one launch
                 Wt = m.weight.detach()
-                w.sigma = sigma_of(m)
                 w.bias = m.bias.detach() if m.bias is not None else None
+                w.sigma = w.src = w.norms = None
+                if isinstance(m, _LOP):
+                    # group norms (and the `scale` buffer, as compute_weight() writes it), then W / max(1, n_k/coeff)
+                    w.src = Wt
+                    w.norms = ops.lop_norms(Wt, m.max_across_dim, ops.lop_norm_type(m.norm_type), scale_out=m.scale)
+                else:
+                    w.sigma = sigma_of(m)
                 cout, cin = Wt.shape[0], Wt.shape[1]
-                if isinstance(m, InducedNormLinear) or m.kernel_size == (1, 1):
+                if isinstance(m, _LINEAR) or m.kernel_size == (1, 1):
                     w.kind, w.cin, w.cout, w.a_type, kind = 'mm', cin, cout, True, 0
                     fshape, bshape = (cout, cin), (cin, cout)
                 else:
@@ -273,8 +291,16 @@ class BranchProgram(object):
                 tc_b = self._use_tc(M, bshape[0], _round_up(bshape[1], 32))
                 fshape = (fshape[0], _round_up(fshape[1], 32) if tc_f else fshape[1])
                 bshape = (bshape[0], _round_up(bshape[1], 32) if tc_b else bshape[1])
-                w.fwd, w.fwd_split, w.bwd, w.bwd_split = ops.prep_weights(Wt, w.sigma, m.coeff, kind, fshape, tc_f,
-                                                                          bshape, tc_b)
+                # effective weight in every layout the kernels consume: one launch
+                if w.norms is not None:
+                    group = (ops.LOP_ROW if m.max_across_dim == 0 else ops.LOP_COL) if m.local_constraint \
+                        else ops.LOP_ONE
+                    w.fwd, w.fwd_split, w.bwd, w.bwd_split = ops.prep_weights_lop(
+                        Wt, w.norms if m.local_constraint else w.norms[-1:], group, m.coeff, kind, fshape, tc_f,
+                        bshape, tc_b)
+                else:
+                    w.fwd, w.fwd_split, w.bwd, w.bwd_split = ops.prep_weights(Wt, w.sigma, m.coeff, kind, fshape,
+                                                                              tc_f, bshape, tc_b)
                 w.fwd_k, w.bwd_k = fshape[1], bshape[1]
                 ws.append(w)
         self._key, self._weights = key, ws
@@ -884,11 +910,18 @@ class BranchProgram(object):
 
     def _finish_param_grads(self, ws, wbars, bbars, betabars):
         """Chain the effective-weight gradients through the spectral rescale W / max(1, sigma/coeff)
-        (mixed_lipschitz.py:125-131: differentiable through sigma with u, v constant) and order
-        everything like nnet.parameters()."""
+        (mixed_lipschitz.py:125-131: differentiable through sigma with u, v constant) or a Lop layer's rescale by its
+        group norms (lipschitz.py:72-79), and order everything like nnet.parameters()."""
         by_id = {}
         for i, (act, m) in enumerate(self.stages):
-            if wbars[i] is not None:
+            if wbars[i] is not None and ws[i].norms is not None:
+                w, Wbar = ws[i], wbars[i]
+                Wbar = Wbar if Wbar.stride(-1) == 1 else Wbar.contiguous()
+                kind = 0 if w.kind == 'mm' else (1 if w.a_type else 2)
+                by_id[id(m.weight)] = ops.lop_scale_grad_layout(
+                    Wbar, kind, w.cout, w.cin, w.src, w.norms, m.coeff, m.max_across_dim,
+                    ops.lop_norm_type(m.norm_type), m.local_constraint).view(m.weight.shape)
+            elif wbars[i] is not None:
                 w, Wbar = ws[i], wbars[i]
                 W = m.weight.detach()
                 D = self._D_static[id(m)] if self._D_static is not None else m.sigma_gradient()
@@ -967,8 +1000,9 @@ class BranchProgram(object):
     # the deeper scales (and for the MLP flows) the GPU finishes them faster than Python can issue them, so after
     # SWEEP_GRAPHS['warmup'] eager calls a sweep is captured once into a CUDA graph over STATIC copies of everything
     # it reads that changes between steps (saved pre-activations, the incoming vectors, the prepared weight planes,
-    # softplus(beta), sigma and d sigma / d W), and every later call is: one multi-tensor copy into the static
-    # inputs, one graph launch, one multi-tensor copy of the results out of the graph's private pool.
+    # softplus(beta), sigma and d sigma / d W, a Lop layer's raw weight and group norms), and every later call is: one
+    # multi-tensor copy into the static inputs, one graph launch, one multi-tensor copy of the results out of the
+    # graph's private pool.
     def _graphable(self, saved, like):
         # MLP flows: the row count of the batched sweep follows the roulette draw of every step (n-fold batch), so a
         # program collects one graph per distinct n (a handful: n = exact terms + a geometric draw); they share one
@@ -988,11 +1022,12 @@ class BranchProgram(object):
         dyn = [saved.rows] + [p for p in saved.pres if p is not None and p is not saved.rows]
         dyn += [v for v in vecs if v is not None]
         for w in ws:
-            dyn += [w.fwd, w.bwd, w.sigma]
+            # what the gradient chain reads: sigma (and d sigma / d W below), or the raw weight and its group norms
+            dyn += [w.fwd, w.bwd] + ([w.sigma] if w.norms is None else [w.src, w.norms])
             dyn += list(w.fwd_split) if w.fwd_split is not None else []
             dyn += list(w.bwd_split) if w.bwd_split is not None else []
         dyn += [a._beta for a in self._acts() if a is not None and a.beta_sp() is not None]
-        dyn += [m.sigma_gradient() for _, m in self.stages]
+        dyn += [m.sigma_gradient() for _, m in self.stages if not isinstance(m, _LOP)]
         return dyn, ws
 
     def _graphed(self, kind, saved, vecs, flags):
@@ -1055,7 +1090,7 @@ class BranchProgram(object):
             w2 = _Weights()
             for name in _Weights.__slots__:
                 setattr(w2, name, getattr(w, name, None))
-            w2.fwd, w2.bwd, w2.sigma = T(w.fwd), T(w.bwd), T(w.sigma)
+            w2.fwd, w2.bwd, w2.sigma, w2.src, w2.norms = T(w.fwd), T(w.bwd), T(w.sigma), T(w.src), T(w.norms)
             w2.fwd_split = tuple(T(t) for t in w.fwd_split) if w.fwd_split is not None else None
             w2.bwd_split = tuple(T(t) for t in w.bwd_split) if w.bwd_split is not None else None
             ws_s.append(w2)
@@ -1069,7 +1104,7 @@ class BranchProgram(object):
             for a in acts:
                 a._beta = T(a._beta)
             self._weights = ws_s
-            self._D_static = {id(m): T(m.sigma_gradient()) for _, m in self.stages}
+            self._D_static = {id(m): T(m.sigma_gradient()) for _, m in self.stages if not isinstance(m, _LOP)}
             ops.GEMM_PROFILE['on'], ops.GEMM_PROFILE['shapes'] = True, {}
             # capture_begin / capture_end directly: the torch.cuda.graph context manager also synchronises the device
             # and EMPTIES the caching allocator, after which the following steps re-allocate everything

@@ -245,16 +245,24 @@ k_sn_scale_grad_layout(const float* __restrict__ Wbar, long long ldw, const floa
 //   kind 0 (linear, 1x1):            fwd[co][ci]                   bwd[ci][co]
 //   kind 1 (3x3, cin <= cout):       fwd[co][(ky,kx,ci)]           bwd[(ky,kx,ci)][co]
 //   kind 2 (3x3, cin >  cout):       fwd[(ky',kx',co)][ci]         bwd[ci][(ky',kx',co)]     taps flipped: ky' = 2-ky
+// The divisor comes from `fac` by group mode (kGroup): kPrepSigma, the induced-norm layers' W / max(1, sigma/coeff);
+// or a closed-form operator norm (LopLinear / LopConv2d, lipschitz.py:72-79) with ratio n * (1/coeff) as torch forms
+// it: one norm for the whole layer (kPrepLopOne), per output row (kPrepLopRow) or per input channel (kPrepLopCol).
 struct PrepOut {
   float* f32;
   float* hi;   // may be null (CUDA-core path: no planes)
   float* lo;
   int N, Kp;   // rows, padded row length
 };
+constexpr int kPrepSigma = -1, kPrepLopOne = 0, kPrepLopRow = 1, kPrepLopCol = 2;
+template <int kGroup>
 __global__ void __launch_bounds__(256)
-k_prep_weights(const float* __restrict__ W, const float* __restrict__ sigma, float coeff, int kind, int cout,
+k_prep_weights(const float* __restrict__ W, const float* __restrict__ fac, float coeff, int kind, int cout,
                int cin, PrepOut fwd, PrepOut bwd) {
-  const float factor = fmaxf(1.f, __ldg(sigma) / coeff);
+  const float rcoeff = 1.f / coeff;
+  float factor = 1.f;
+  if (kGroup == kPrepSigma) factor = fmaxf(1.f, __ldg(fac) / coeff);
+  if (kGroup == kPrepLopOne) factor = fmaxf(1.f, __ldg(fac) * rcoeff);
   const int nf = fwd.N * fwd.Kp, nb = bwd.N * bwd.Kp;
   const int taps = kind == 0 ? 1 : 9;
   for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < nf + nb; i += gridDim.x * blockDim.x) {
@@ -272,7 +280,10 @@ k_prep_weights(const float* __restrict__ W, const float* __restrict__ sigma, flo
       if (is_fwd) { if (k < cin) { const int t = r / cout; co = r - t * cout, ci = k, tap = 8 - t; } }
       else { if (k < 9 * cout) { const int t = k / cout; co = k - t * cout, ci = r, tap = 8 - t; } }
     }
-    const float v = co >= 0 ? W[((long long)co * cin + ci) * taps + tap] / factor : 0.f;
+    float f = factor;
+    if (kGroup == kPrepLopRow && co >= 0) f = fmaxf(1.f, __ldg(fac + co) * rcoeff);
+    if (kGroup == kPrepLopCol && co >= 0) f = fmaxf(1.f, __ldg(fac + ci) * rcoeff);
+    const float v = co >= 0 ? W[((long long)co * cin + ci) * taps + tap] / f : 0.f;
     o.f32[j] = v;
     if (o.hi != nullptr) {
       uint32_t hb;
@@ -283,6 +294,132 @@ k_prep_weights(const float* __restrict__ W, const float* __restrict__ sigma, flo
   }
 }
 
+
+// ---- closed-form operator norms (LopLinear / LopConv2d) -------------------------------------------------------------
+// Group k of a [cout][cin][taps] weight is output row k (axis 0) or input channel k (axis 1).  Norm type 1: sum |w|,
+// 2: sqrt(sum w^2), 3: the SIGNED maximum (the reference's _max_except_dim, lipschitz.py:51).  One warp per group, a
+// fixed lane order and a butterfly: deterministic, no atomics.
+constexpr int kLopGroupsPerCta = 8;
+__device__ __forceinline__ long long lop_elem(int axis, int cin, int taps, int k, int j) {
+  if (axis == 0) return (long long)k * cin * taps + j;
+  const int co = j / taps, t = j - co * taps;
+  return ((long long)co * cin + k) * taps + t;
+}
+__device__ __forceinline__ float warp_max(float v) {
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
+  return v;
+}
+__global__ void __launch_bounds__(32 * kLopGroupsPerCta)
+k_lop_norms(const float* __restrict__ W, int cout, int cin, int taps, int axis, int norm_type,
+            float* __restrict__ norms) {
+  const int k = blockIdx.x * kLopGroupsPerCta + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  const int groups = axis == 0 ? cout : cin, len = (axis == 0 ? cin : cout) * taps;
+  if (k >= groups) return;
+  float acc = norm_type == 3 ? -INFINITY : 0.f;
+  for (int j = lane; j < len; j += 32) {
+    const float w = __ldg(W + lop_elem(axis, cin, taps, k, j));
+    acc = norm_type == 3 ? fmaxf(acc, w) : (norm_type == 1 ? acc + fabsf(w) : fmaf(w, w, acc));
+  }
+  acc = norm_type == 3 ? warp_max(acc) : warp_sum(acc);
+  if (lane == 0) norms[k] = norm_type == 2 ? sqrtf(acc) : acc;
+}
+// norms[groups] = the largest group norm (the global constraint's norm and the `scale` buffer, lipschitz.py:74-77)
+__global__ void __launch_bounds__(1024)
+k_lop_norm_max(float* __restrict__ norms, int groups, float* __restrict__ scale_out) {
+  __shared__ float scratch[32];
+  float m = -INFINITY;
+  for (int k = threadIdx.x; k < groups; k += 1024) m = fmaxf(m, norms[k]);
+  m = warp_max(m);
+  if ((threadIdx.x & 31) == 0) scratch[threadIdx.x >> 5] = m;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    float t = scratch[0];
+    for (int w = 1; w < 32; ++w) t = fmaxf(t, scratch[w]);
+    norms[groups] = t;
+    if (scale_out != nullptr) scale_out[0] = t;
+  }
+}
+
+// Gradient chain of W / f_k, f_k = max(1, n_k/coeff), from the GEMM-layout gradient (read through wbar_index):
+//   dL/dW = Gbar/f_k - c_k t_k / (coeff f_k^2) dn_k/dW,   t_k = sum_{group k} Gbar W,
+// c_k = 1 above the bound, 1/2 exactly at it (torch.max's even split), 0 below.  Phase 1: t_k and, for the signed
+// maximum, the number of entries equal to n_k (amax's backward splits evenly among them), one warp per group.
+__global__ void __launch_bounds__(32 * kLopGroupsPerCta)
+k_lop_grad_dot(const float* __restrict__ Wbar, long long ldw, const float* __restrict__ W,
+               const float* __restrict__ norms, int kind, int cout, int cin, int axis, float* __restrict__ ws) {
+  const int taps = kind == 0 ? 1 : 9;
+  const int k = blockIdx.x * kLopGroupsPerCta + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+  const int groups = axis == 0 ? cout : cin, len = (axis == 0 ? cin : cout) * taps;
+  if (k >= groups) return;
+  const float nk = norms[k];
+  float t = 0.f, ties = 0.f;
+  for (int j = lane; j < len; j += 32) {
+    const long long i = lop_elem(axis, cin, taps, k, j);
+    const float w = __ldg(W + i);
+    t = fmaf(Wbar[wbar_index(kind, cout, cin, ldw, i)], w, t);
+    ties += w == nk ? 1.f : 0.f;
+  }
+  t = warp_sum(t);
+  ties = warp_sum(ties);
+  if (lane == 0) {
+    ws[k] = t;
+    ws[groups + k] = ties;
+  }
+}
+// Phase 2, elementwise.  local = 0: one factor from the largest norm N = norms[groups]; t = sum_k t_k and the
+// derivative of N is split evenly among the groups whose norm equals N (every block sums the same values in the
+// same order).
+__global__ void __launch_bounds__(256)
+k_lop_scale_grad_layout(const float* __restrict__ Wbar, long long ldw, const float* __restrict__ W,
+                        const float* __restrict__ norms, const float* __restrict__ ws, float coeff, int kind,
+                        int cout, int cin, int axis, int norm_type, int local, float* __restrict__ out) {
+  const int taps = kind == 0 ? 1 : 9;
+  const int groups = axis == 0 ? cout : cin;
+  const float rcoeff = 1.f / coeff;
+  __shared__ float red[2][256];
+  float t_all = 0.f, n_tied = 0.f;
+  if (!local) {
+    const float N = norms[groups];
+    float a = 0.f, b = 0.f;
+    for (int k = threadIdx.x; k < groups; k += 256) {
+      a += ws[k];
+      b += norms[k] == N ? 1.f : 0.f;
+    }
+    red[0][threadIdx.x] = a;
+    red[1][threadIdx.x] = b;
+    __syncthreads();
+    for (int s = 128; s > 0; s >>= 1) {
+      if (threadIdx.x < s) {
+        red[0][threadIdx.x] += red[0][threadIdx.x + s];
+        red[1][threadIdx.x] += red[1][threadIdx.x + s];
+      }
+      __syncthreads();
+    }
+    t_all = red[0][0];
+    n_tied = red[1][0];
+  }
+  const long long n = (long long)cout * cin * taps;
+  for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < n; i += (long long)gridDim.x * blockDim.x) {
+    const int co = (int)(i / ((long long)cin * taps)), ci = (int)((i / taps) % cin);
+    const int k = axis == 0 ? co : ci;
+    const float nk = norms[k], N = local ? nk : norms[groups];
+    const float ratio = N * rcoeff;
+    const float f = fmaxf(1.f, ratio);
+    const float g = Wbar[wbar_index(kind, cout, cin, ldw, i)];
+    float r = g / f;
+    const float c = ratio > 1.f ? 1.f : (ratio == 1.f ? 0.5f : 0.f);
+    if (c != 0.f && nk == N) {
+      const float w = W[i];
+      float dn = norm_type == 1 ? (w > 0.f ? 1.f : (w < 0.f ? -1.f : 0.f))
+                                : (norm_type == 2 ? w / nk : (w == nk ? 1.f / ws[groups + k] : 0.f));
+      if (!local) dn /= n_tied;
+      const float t = local ? ws[k] : t_all;
+      r -= c * t / (coeff * f * f) * dn;
+    }
+    out[i] = r;
+  }
+}
 }  // namespace impflow
 
 using namespace impflow;
@@ -299,8 +436,65 @@ extern "C" int impflow_prep_weights(const float* W, const float* sigma, float co
   PrepOut f{fwd, fwd_hi, fwd_lo, fwd_rows, fwd_k}, b{bwd, bwd_hi, bwd_lo, bwd_rows, bwd_k};
   long long blocks = (total + 255) / 256;
   if (blocks > 148 * 8) blocks = 148 * 8;
-  k_prep_weights<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(W, sigma, coeff, kind, cout, cin, f, b);
+  k_prep_weights<kPrepSigma><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(W, sigma, coeff, kind, cout, cin, f, b);
   return check_launch("k_prep_weights");
+}
+
+extern "C" int impflow_prep_weights_lop(const float* W, const float* norms, int group, float coeff, int kind,
+                                        int cout, int cin, float* fwd, float* fwd_hi, float* fwd_lo, int fwd_rows,
+                                        int fwd_k, float* bwd, float* bwd_hi, float* bwd_lo, int bwd_rows, int bwd_k,
+                                        void* stream) {
+  IMPFLOW_REQUIRE(kind >= 0 && kind <= 2 && cout >= 1 && cin >= 1, "prep_weights_lop: bad layer (kind=%d)", kind);
+  IMPFLOW_REQUIRE(group >= 0 && group <= 2, "prep_weights_lop: bad group mode %d", group);
+  IMPFLOW_REQUIRE(norms != nullptr && fwd != nullptr && bwd != nullptr, "prep_weights_lop: operands missing");
+  IMPFLOW_REQUIRE((fwd_hi == nullptr) == (fwd_lo == nullptr) && (bwd_hi == nullptr) == (bwd_lo == nullptr),
+                  "prep_weights_lop: planes come in pairs");
+  const long long total = (long long)fwd_rows * fwd_k + (long long)bwd_rows * bwd_k;
+  IMPFLOW_REQUIRE(total < (1LL << 31), "prep_weights_lop: layer too large");
+  PrepOut f{fwd, fwd_hi, fwd_lo, fwd_rows, fwd_k}, b{bwd, bwd_hi, bwd_lo, bwd_rows, bwd_k};
+  long long blocks = (total + 255) / 256;
+  if (blocks > 148 * 8) blocks = 148 * 8;
+  cudaStream_t s = (cudaStream_t)stream;
+  if (group == kPrepLopOne)
+    k_prep_weights<kPrepLopOne><<<(int)blocks, 256, 0, s>>>(W, norms, coeff, kind, cout, cin, f, b);
+  else if (group == kPrepLopRow)
+    k_prep_weights<kPrepLopRow><<<(int)blocks, 256, 0, s>>>(W, norms, coeff, kind, cout, cin, f, b);
+  else
+    k_prep_weights<kPrepLopCol><<<(int)blocks, 256, 0, s>>>(W, norms, coeff, kind, cout, cin, f, b);
+  return check_launch("k_prep_weights");
+}
+
+extern "C" int impflow_lop_norms(const float* W, int cout, int cin, int taps, int axis, int norm_type, float* norms,
+                                 float* scale_out, void* stream) {
+  IMPFLOW_REQUIRE(W != nullptr && norms != nullptr && cout >= 1 && cin >= 1 && taps >= 1, "lop_norms: bad layer");
+  IMPFLOW_REQUIRE((axis == 0 || axis == 1) && norm_type >= 1 && norm_type <= 3,
+                  "lop_norms: axis %d / norm type %d", axis, norm_type);
+  const int groups = axis == 0 ? cout : cin;
+  k_lop_norms<<<(groups + kLopGroupsPerCta - 1) / kLopGroupsPerCta, 32 * kLopGroupsPerCta, 0, (cudaStream_t)stream>>>(
+      W, cout, cin, taps, axis, norm_type, norms);
+  if (check_launch("k_lop_norms")) return -1;
+  k_lop_norm_max<<<1, 1024, 0, (cudaStream_t)stream>>>(norms, groups, scale_out);
+  return check_launch("k_lop_norm_max");
+}
+
+extern "C" int impflow_lop_scale_grad_layout(const float* Wbar, long long ldw, const float* W, const float* norms,
+                                             float coeff, int kind, int cout, int cin, int axis, int norm_type,
+                                             int local, float* out, float* ws, void* stream) {
+  IMPFLOW_REQUIRE(kind >= 0 && kind <= 2 && cout >= 1 && cin >= 1, "lop_scale_grad_layout: bad layer description");
+  IMPFLOW_REQUIRE((axis == 0 || axis == 1) && norm_type >= 1 && norm_type <= 3,
+                  "lop_scale_grad_layout: axis %d / norm type %d", axis, norm_type);
+  IMPFLOW_REQUIRE(ws != nullptr && norms != nullptr, "lop_scale_grad_layout: workspace or norms missing");
+  const int groups = axis == 0 ? cout : cin;
+  cudaStream_t s = (cudaStream_t)stream;
+  k_lop_grad_dot<<<(groups + kLopGroupsPerCta - 1) / kLopGroupsPerCta, 32 * kLopGroupsPerCta, 0, s>>>(
+      Wbar, ldw, W, norms, kind, cout, cin, axis, ws);
+  if (check_launch("k_lop_grad_dot")) return -1;
+  const long long n = (long long)cout * cin * (kind == 0 ? 1 : 9);
+  long long blocks = (n + 255) / 256;
+  if (blocks > 148 * 4) blocks = 148 * 4;
+  k_lop_scale_grad_layout<<<(int)blocks, 256, 0, s>>>(Wbar, ldw, W, norms, ws, coeff, kind, cout, cin, axis, norm_type,
+                                                     local, out);
+  return check_launch("k_lop_scale_grad_layout");
 }
 
 extern "C" int impflow_sn_scale(const float* W, const float* sigma, float coeff, float* out, float* scale_out,

@@ -638,21 +638,59 @@ def sn_rescale(W, sigma, coeff, scale_out=None):
     return out
 
 
-def prep_weights(W, sigma, coeff, kind, fwd_shape, fwd_planes, bwd_shape, bwd_planes):
-    """Rescaled weight in the forward / transposed GEMM layouts (+ hi/lo planes) in one launch; see
-    impflow_prep_weights.  *_shape = (rows, padded K)."""
-    W = W.contiguous()
+def _prep_layouts(W, fwd_shape, fwd_planes, bwd_shape, bwd_planes):
+    """Output tensors of the weight-preparation launch and the layout arguments after the scale operands."""
     dev = W.device
     mk = lambda shp: torch.empty(shp[0], shp[1], device=dev, dtype=torch.float32)
     f, b = mk(fwd_shape), mk(bwd_shape)
     fs = (mk(fwd_shape), mk(fwd_shape)) if fwd_planes else None
     bs = (mk(bwd_shape), mk(bwd_shape)) if bwd_planes else None
-    _cabi.check(_lib().impflow_prep_weights(
-        _cabi.ptr(W), _cabi.ptr(sigma), float(coeff), kind, W.shape[0], W.shape[1], _cabi.ptr(f),
-        _cabi.ptr(fs[0] if fs else None, 'fh', True), _cabi.ptr(fs[1] if fs else None, 'fl', True), fwd_shape[0],
-        fwd_shape[1], _cabi.ptr(b), _cabi.ptr(bs[0] if bs else None, 'bh', True),
-        _cabi.ptr(bs[1] if bs else None, 'bl', True), bwd_shape[0], bwd_shape[1], _cabi.stream()), 'prep_weights')
-    return f, fs, b, bs
+    args = (W.shape[0], W.shape[1], _cabi.ptr(f), _cabi.ptr(fs[0] if fs else None, 'fh', True),
+            _cabi.ptr(fs[1] if fs else None, 'fl', True), fwd_shape[0], fwd_shape[1], _cabi.ptr(b),
+            _cabi.ptr(bs[0] if bs else None, 'bh', True), _cabi.ptr(bs[1] if bs else None, 'bl', True), bwd_shape[0],
+            bwd_shape[1], _cabi.stream())
+    return (f, fs, b, bs), args
+
+
+def prep_weights(W, sigma, coeff, kind, fwd_shape, fwd_planes, bwd_shape, bwd_planes):
+    """Rescaled weight in the forward / transposed GEMM layouts (+ hi/lo planes) in one launch; see
+    impflow_prep_weights.  *_shape = (rows, padded K)."""
+    W = W.contiguous()
+    out, args = _prep_layouts(W, fwd_shape, fwd_planes, bwd_shape, bwd_planes)
+    _cabi.check(_lib().impflow_prep_weights(_cabi.ptr(W), _cabi.ptr(sigma), float(coeff), kind, *args),
+                'prep_weights')
+    return out
+
+
+# Lop layers (LopLinear / LopConv2d): norm types of impflow_lop_norms and group modes of impflow_prep_weights_lop
+LOP_L1, LOP_L2, LOP_MAX = 1, 2, 3
+LOP_ONE, LOP_ROW, LOP_COL = 0, 1, 2
+
+
+def lop_norm_type(norm_type):
+    return {1: LOP_L1, 2: LOP_L2, float('inf'): LOP_MAX}[norm_type]
+
+
+def lop_norms(W, axis, norm_type, scale_out=None):
+    """Group norms of a Lop layer's weight (module layout), followed by their maximum: (groups + 1,) device tensor;
+    scale_out (the layer's `scale` buffer) receives the maximum too.  See impflow_lop_norms."""
+    W = W.contiguous()
+    taps = W[0, 0].numel()
+    norms = torch.empty((W.shape[0] if axis == 0 else W.shape[1]) + 1, device=W.device, dtype=torch.float32)
+    _cabi.check(_lib().impflow_lop_norms(_cabi.ptr(W), W.shape[0], W.shape[1], taps, axis, norm_type,
+                                         _cabi.ptr(norms), _cabi.ptr(scale_out, 'scale', True), _cabi.stream()),
+                'lop_norms')
+    return norms
+
+
+def prep_weights_lop(W, norms, group, coeff, kind, fwd_shape, fwd_planes, bwd_shape, bwd_planes):
+    """prep_weights for a Lop layer: W / max(1, n/coeff) with n one norm (group LOP_ONE: norms[0]) or the norm of
+    each output row / input channel (LOP_ROW / LOP_COL); see impflow_prep_weights_lop."""
+    W = W.contiguous()
+    out, args = _prep_layouts(W, fwd_shape, fwd_planes, bwd_shape, bwd_planes)
+    _cabi.check(_lib().impflow_prep_weights_lop(_cabi.ptr(W), _cabi.ptr(norms), group, float(coeff), kind, *args),
+                'prep_weights_lop')
+    return out
 
 
 def _flat_dot(a, b):
@@ -696,6 +734,19 @@ def sn_scale_grad_layout(Wbar, kind, cout, cin, W, D, sigma, coeff):
     _cabi.check(_lib().impflow_sn_scale_grad_layout(_cabi.ptr(Wbar), Wbar.stride(0), _cabi.ptr(W), _cabi.ptr(D),
                                                     _cabi.ptr(sigma), float(coeff), kind, cout, cin, _cabi.ptr(out),
                                                     _cabi.ptr(ws), _cabi.stream()), 'sn_scale_grad_layout')
+    return out
+
+
+def lop_scale_grad_layout(Wbar, kind, cout, cin, W, norms, coeff, axis, norm_type, local):
+    """dL/dW of a Lop layer from dL/dW_eff in the GEMM layout (kind 0 / 1 / 2 as in sn_scale_grad_layout), in the
+    module's weight layout; norms as lop_norms returned them.  See impflow_lop_scale_grad_layout."""
+    assert Wbar.stride(-1) == 1 and W.is_contiguous()
+    out = torch.empty_like(W)
+    ws = torch.empty(2 * (cout if axis == 0 else cin), device=W.device, dtype=torch.float32)
+    _cabi.check(_lib().impflow_lop_scale_grad_layout(_cabi.ptr(Wbar), Wbar.stride(0), _cabi.ptr(W), _cabi.ptr(norms),
+                                                     float(coeff), kind, cout, cin, axis, norm_type, int(bool(local)),
+                                                     _cabi.ptr(out), _cabi.ptr(ws), _cabi.stream()),
+                'lop_scale_grad_layout')
     return out
 
 

@@ -491,6 +491,27 @@ int impflow_sn_scale_grad(const float* G, const float* D, const float* sigma, co
 int impflow_sn_scale_grad_layout(const float* Wbar, long long ldw, const float* W, const float* D, const float* sigma,
                                  float coeff, int kind, int cout, int cin, float* out, float* ws, void* stream);
 
+/* Closed-form operator norms of a LopLinear / LopConv2d weight W [cout][cin][taps] (lipschitz.py:46-79): per output
+ * row (axis 0) or per input channel (axis 1), norm_type 1 = sum |w|, 2 = sqrt(sum w^2), 3 = the signed maximum
+ * (the reference's _max_except_dim).  norms: groups + 1 floats; norms[groups] receives the largest group norm, as
+ * does scale_out[0] when given (the layer's `scale` buffer).  Fixed reduction order, no atomics. */
+int impflow_lop_norms(const float* W, int cout, int cin, int taps, int axis, int norm_type, float* norms,
+                      float* scale_out, void* stream);
+/* impflow_prep_weights for a Lop layer: the same layouts and planes of W / max(1, n * (1/coeff)) with n = norms[0]
+ * (group 0: one norm, local_constraint off), norms[co] (group 1: per output row) or norms[ci] (group 2: per input
+ * channel). */
+int impflow_prep_weights_lop(const float* W, const float* norms, int group, float coeff, int kind, int cout, int cin,
+                             float* fwd, float* fwd_hi, float* fwd_lo, int fwd_rows, int fwd_k, float* bwd,
+                             float* bwd_hi, float* bwd_lo, int bwd_rows, int bwd_k, void* stream);
+/* Gradient of a Lop layer's weight from dL/dW_eff in the GEMM layout of impflow_sn_scale_grad_layout (kind, ldw):
+ * dL/dW = Gbar/f_k - c_k t_k / (coeff f_k^2) dn_k/dW with t_k = sum over group k of Gbar W, c_k = 1 above the bound,
+ * 1/2 exactly at it, 0 below; dn_k/dW as torch autograd forms it (sign(W); W / n_k; the signed maximum split evenly
+ * among its ties; local = 0: one norm, split evenly among the tied groups).  norms as impflow_lop_norms wrote them;
+ * out in the module layout; ws: 2 * groups floats.  Two launches, deterministic. */
+int impflow_lop_scale_grad_layout(const float* Wbar, long long ldw, const float* W, const float* norms, float coeff,
+                                  int kind, int cout, int cin, int axis, int norm_type, int local, float* out,
+                                  float* ws, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
